@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the flat-search hot path (BASELINE.json: queries/s at 1024-d, k=100).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config C4 of BASELINE.json / SURVEY.md section 8d): synthetic 10M x 1024 fp32
@@ -28,6 +28,8 @@ Legs, all in one JSON line printed by rank 0:
   cpu_baseline  blocked sgemm + top-k on the host cores (bounded sample, scaled by N)
 --impl reference times the CPU implementation only (see oracle/cpu_baseline.py).
 --config c2|c3 selects the rescoring-heavy all-vs-all stand-ins of BASELINE.json's configs 2 and 3 (k = 1000).
+--dump-outputs DIR writes the (D, I) of the last timed step as DIR/D.npy and DIR/I.npy (see dump_outputs); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -77,7 +79,14 @@ def parse():
     ap.add_argument("--parity-queries", type=int, default=256)
     ap.add_argument("--param", action="append", default=[], metavar="NAME=VALUE",
                     help="knn_index_set_param on every rank's index (A/B experiments; results never depend on it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (D, I) of the last timed step as DIR/D.npy (float32) and DIR/I.npy (float64), "
+                         "at most 64 MB together (a fixed, seeded sample of query rows when the whole result is larger)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm keeps only its timings)")
     if args.config == "c2":
         args.nb, args.nq, args.k, args.all_vs_all = 14_433, 14_433, 1000, True
     elif args.config == "c3":
@@ -296,6 +305,30 @@ def compare_with_fp64(D_s, I_s, best_s, best_i, k, d):
             "tau": tau, "rtol_D": 1e-5, "ok": bool(n_beyond == 0 and dup == 0 and max_rel <= 1e-5)}
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, D, I, limit=DUMP_LIMIT_BYTES):
+    """Writes the search result (D, I) as out_dir/D.npy (float32) and out_dir/I.npy (float64, exact for ids below
+    2**53), at most `limit` bytes together.  A larger result is cut to a sample of query rows drawn with a fixed seed
+    (sorted, the same rows in both files), so two builds given the same arguments write the same rows.  Returns the
+    number of query rows written."""
+    import numpy as np
+    import torch
+
+    nq, k = D.shape
+    fit = max(1, (limit - 1024) // (k * (4 + 8)))  # 1024 bytes: room for the two .npy headers
+    if fit < nq:
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=fit, replace=False))
+        sel = torch.from_numpy(rows).to(D.device)
+        D, I = D[sel], I[sel]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "D.npy", D.cpu().numpy().astype(np.float32, copy=False))
+    np.save(out / "I.npy", I.cpu().numpy().astype(np.float64))
+    return int(D.shape[0])
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -447,6 +480,7 @@ def main():
     value = args.nq * args.steps / (ms / 1e3)
     by_rank_value = dict(by_rank)  # per-rank step / GEMM time of the `value` leg (chip-to-chip spread under the power cap)
     D, I = last["DI"]  # result of the last timed step
+    dumped_rows = dump_outputs(args.dump_outputs, D, I) if args.dump_outputs and rank == 0 else None
     search_path = int(index.local.stat("path"))
     fmt_names = {1: "bf16", 2: "fp16"}
     fmt = fmt_names[int(index.local.stat("shadow_fmt"))]
@@ -569,6 +603,7 @@ def main():
             "query_share_by_group": ([round(w / sum(index.group_weights), 4) for w in index.group_weights]
                                      if Q > 1 and getattr(index, "group_weights", None) else None),
             "overlap_finish": not args.no_overlap, "params": args.param or None, "autotune_query_shares": bool(Q > 1 and not args.no_autotune),
+            "dumped_query_rows": dumped_rows,
         }
         print(json.dumps(line), flush=True)
     if world > 1:

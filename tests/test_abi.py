@@ -1,7 +1,11 @@
 """CPU tests of the drop-in boundary: the C-ABI library loads, exports every symbol that
 include/knn_b200.h declares, and fails loudly (no CPU fallback) when there is no device."""
 import ctypes
+import os
 import re
+import subprocess
+import sys
+import textwrap
 from pathlib import Path
 
 import numpy as np
@@ -63,16 +67,20 @@ def test_argument_errors_before_any_device_work():
 
 
 def test_fails_loudly_without_a_device():
-    import torch
-
-    import knn_b200
-
-    if torch.cuda.is_available():
-        pytest.skip("a CUDA device is present")
-    with pytest.raises(knn_b200._lib.KnnError, match="no CPU fallback"):
-        knn_b200.IndexFlat(16, 0)
-    with pytest.raises(knn_b200._lib.KnnError):
-        knn_b200.normalize_L2(np.ones((2, 4), np.float32))
+    """In a child process with every CUDA device hidden, so that a machine with a GPU checks it too."""
+    script = textwrap.dedent(f"""
+        import sys
+        sys.path.insert(0, {str(REPO / "knn-for-homology_b200")!r})
+        import numpy as np
+        import pytest
+        import knn_b200
+        with pytest.raises(knn_b200._lib.KnnError, match="no CPU fallback"):
+            knn_b200.IndexFlat(16, 0)
+        with pytest.raises(knn_b200._lib.KnnError):
+            knn_b200.normalize_L2(np.ones((2, 4), np.float32))
+        """)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    subprocess.run([sys.executable, "-c", script], env=env, check=True, timeout=300)
 
 
 def test_missing_library_is_an_import_error(monkeypatch, tmp_path):
