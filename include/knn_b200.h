@@ -90,7 +90,8 @@ int knn_index_search_dev(knn_index* idx, int64_t nq, const float* xq_dev, int64_
 
 /* Two-phase search for a row-sharded database (new; see DESIGN.md section 6).  Phase 1 runs the
  * tensor-core filter over this shard and writes lower_dev[q], a lower bound of the TRUE k-th best score
- * of query q within the shard (-FLT_MAX when the shard cannot offer one), and optionally lower_j_dev[q],
+ * of query q within the shard (L2: of the key 2<x,y> - |y|^2, larger = closer, exact arithmetic)
+ * (-FLT_MAX when the shard cannot offer one), and optionally lower_j_dev[q],
  * the same for the j-th best (1 <= j <= k; pass NULL to skip).  The caller combines the bounds of all G
  * shards - element-wise MAX of lower, and with j = ceil(k / G) element-wise MIN of lower_j (every shard holds
  * j rows at or above it, G*j >= k in total), e.g. two NCCL all-reduces - takes the larger of the two and

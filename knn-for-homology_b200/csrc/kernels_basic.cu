@@ -162,17 +162,30 @@ __global__ void __launch_bounds__(kBlock) ingest_rows_kernel(const float* __rest
 // approx score is the 16-bit x 16-bit -> fp32 tensor-core inner product (DESIGN.md "error bound"):
 //   |<x^,y^> - <x,y>| <= |dx||y| + |x||dy| + |dx||dy|      (Cauchy-Schwarz, dx = x^ - x)
 // plus a slack of dp * 2^-22 * |x||y| for the fp32 accumulation inside the MMA and the rerank.
+// L2 compares keys 2<x,y> - |y|^2: the inner-product bound doubles, and fp32 roundings of order ulp(|y|^2) that no
+// inner-product term sees are added, in units U = 2^-24 (|x|^2 + max|y|^2):
+//   |y|^2 itself (ingest: a lane chains dp/32 FMAs, then 5 butterfly adds)            dp/32 + 5
+//   the key fl(2 acc - |y|^2), |key| <= |x|^2 + 2|y|^2                                  2
+//   the rescored distance fl(fl(|x|^2 + |y|^2) - 2a), |D| <= 2 (|x|^2 + |y|^2)          1 + 2
+//   threshold = k-th key - 2 eps, lower = threshold + eps, lower - eps (values <= 2U)   3 x 2
+// c(dp) = dp/32 + 16.  Negligible for normalised data (~6e-6 at dp = 1024 against eps ~1e-3); what it covers
+// dominates when |x| << |y| or the data is 16-bit exact (eps = the slack alone), e.g. |y| / |x| = 4000 at dp = 64.
 __global__ void query_eps_kernel(const float* __restrict__ xnorm2, const float* dnorm2, int64_t nq, int dp,
                                  const DbStats* __restrict__ stats, int metric, float* eps) {  // dnorm2 may alias eps
     int64_t q = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (q >= nq) return;
-    const float ymax = sqrtf(__uint_as_float(stats->max_norm2));
+    const float ymax2 = __uint_as_float(stats->max_norm2);
+    const float ymax = sqrtf(ymax2);
     const float dymax = sqrtf(__uint_as_float(stats->max_dnorm2));
-    const float xn = sqrtf(xnorm2[q]);
+    const float xn2 = xnorm2[q];
+    const float xn = sqrtf(xn2);
     const float dx = sqrtf(dnorm2[q]);
     float e = dx * ymax + xn * dymax + dx * dymax + float(dp) * 2.384185791015625e-07f * xn * ymax;
     e *= 1.001f;
-    if (metric == KNN_METRIC_L2) e *= 2.f;  // approx score is 2<x,y> - |y|^2
+    if (metric == KNN_METRIC_L2) {
+        e *= 2.f;  // approx score is 2<x,y> - |y|^2
+        e += (float(dp) * 0.03125f + 16.f) * 5.9604644775390625e-08f * (xn2 + ymax2);
+    }
     if (!(e == e) || e > FLT_MAX) e = FLT_MAX;
     eps[q] = e;
 }
