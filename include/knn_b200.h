@@ -107,7 +107,10 @@ int knn_index_search_finish_dev(knn_index* idx, int64_t nq, const float* xq_dev,
  * with the filter of the next on a second stream (knn_b200/distributed.py does: filter of batch b on the main stream,
  * event, then on a side stream all-reduce of that batch's bounds and finish_batch).
  *   begin         fixes (nq, xq_dev, k) - xq_dev must stay valid until `end` - and returns the number of query batches
- *                 and the rows per batch (the last batch may be shorter);
+ *                 and the rows per batch (the last batch may be shorter).  Both depend on nq and the index's
+ *                 query_batch alone - batch_rows = min(query_batch, nq) rounded up to 256 - never on the shard's size
+ *                 or path, so shards with the same query_batch report identical values and exchange bounds batch by
+ *                 batch (an exact-path shard offers no bound and finishes each batch with the exact scan);
  *   filter_batch  filters batch b and writes its bounds into bounds_dev, a caller-zeroed float array
  *                 [nbatches][2][batch_rows]: [b][0][i] = lower bound of the k-th best true score of query
  *                 b*batch_rows+i in this shard, [b][1][i] = MINUS the bound on the j-th best (j = ceil(k / shards)):

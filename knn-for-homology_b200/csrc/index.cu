@@ -1212,16 +1212,17 @@ static int two_phase_begin(knn_index* ix, int64_t nq, const float* xq_dev, int64
     P.launches0 = g_launches.load();
     P.tensor = ix->ntotal > 0 && use_tensor_path(ix, nq, k);
     ix->last_path = P.tensor ? 2 : 1;
-    if (!P.tensor) {  // exact path: nothing to filter, no bound to offer; one "batch" that finish runs in one go
-        P.qb = nq;
-        P.nbatches = 1;
+    // The batch geometry depends on nq and query_batch alone, never on the path: the shards of one search lay out
+    // their bound slots [batch][shard][2 * rows] from it and exchange bounds batch by batch, so a shard on the exact
+    // path (fewer rows than tensor_min_n or than k, empty, path = 1) must cut the queries exactly as the others do.
+    P.qb = round_up(std::min<int64_t>(ix->query_batch, nq), 256);
+    P.nbatches = (nq + P.qb - 1) / P.qb;
+    if (!P.tensor) {  // exact path: nothing to filter, no bound to offer; finish scans each batch's queries
         P.active = true;
         return KNN_OK;
     }
     KNN_CHECK(prepare_shadow(ix, k, s));
     P.cap = candidate_capacity(k, ix->ntotal, ix->dense_small_db != 0);
-    P.qb = round_up(std::min<int64_t>(ix->query_batch, nq), 256);
-    P.nbatches = (nq + P.qb - 1) / P.qb;
     KNN_CHECK(tensor_ws_ensure(ix->ws2, P.nbatches * P.qb, ix->dp, P.cap));
     KNN_CHECK(ix->overflow.ensure(sizeof(int) * size_t(P.nbatches)));
     KNN_CHECK(ix->ovf_q.ensure(sizeof(int) * size_t(nq)));
@@ -1240,6 +1241,10 @@ static int two_phase_filter_batch(knn_index* ix, int64_t b, float* lower_b, int6
     auto& P = ix->pend;
     const int64_t q0 = b * P.qb;
     const int64_t nb = P.nq - q0 < P.qb ? P.nq - q0 : P.qb;
+    if (lower_j_b && (j < 1 || j > P.k)) {
+        set_error("search_filter: j must be in [1, k]");
+        return KNN_ERR_INVALID;
+    }
     if (!P.tensor) {
         KNN_CHECK(launch_fill_f32(lower_b, nb, -FLT_MAX, s));
         if (lower_j_b) KNN_CHECK(launch_fill_f32(lower_j_b, nb, negate_j ? FLT_MAX : -FLT_MAX, s));
@@ -1249,10 +1254,6 @@ static int two_phase_filter_batch(knn_index* ix, int64_t b, float* lower_b, int6
                                   ix->ovf_q.as<int>() + q0, s));
     KNN_CHECK(launch_export_lower(ix->ws2.thr.as<float>() + q0, ix->ws2.eps.as<float>() + q0, nb, lower_b, s));
     if (lower_j_b) {
-        if (j < 1 || j > P.k) {
-            set_error("search_filter: j must be in [1, k]");
-            return KNN_ERR_INVALID;
-        }
         KNN_CHECK(launch_kth_lower(filter_state(ix->ws2, q0, P.cap), ix->ws2.eps.as<float>() + q0, nb, int(j), negate_j, lower_j_b, s));
     }
     return KNN_OK;
@@ -1264,8 +1265,11 @@ static int two_phase_finish_batch(knn_index* ix, int64_t b, const float* lower_b
     const int64_t q0 = b * P.qb;
     const int64_t nb = P.nq - q0 < P.qb ? P.nq - q0 : P.qb;
     if (!P.tensor) {
+        // rows [q0, q0 + nb) by the exact scan (padding when the shard is empty).  A slice of the queries takes the exact
+        // path whenever all of them do.  The scan uses the index's shared scratch (xq_f32, scores, lists): every batch of
+        // an exact shard must be finished on the same stream.
         const long long l0 = P.launches0;
-        KNN_CHECK(search_dev_impl(ix, P.nq, P.xq, P.k, D_dev, I_dev, id_base, s));
+        KNN_CHECK(search_dev_impl(ix, nb, P.xq + q0 * ix->d, P.k, D_dev + q0 * P.k, I_dev + q0 * P.k, id_base, s));
         P.launches0 = l0;
         return KNN_OK;
     }

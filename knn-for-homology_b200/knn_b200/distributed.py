@@ -134,11 +134,13 @@ class BoundsExchange:
     """Per-batch MAX-reduction of the two-phase search's bounds over peer memory (knn_bounds_push_peer_dev /
     knn_bounds_wait_max_dev).  Every rank owns slots [batch][rank][2 * rows] floats and flags [batch][rank]; a search is
     one epoch.  Two searches are separated by the barriers of the result merge, so slots are never overwritten while a
-    slower rank still reads them.  All methods are collective in the sense that every rank calls them in the same order."""
+    slower rank still reads them.  All methods are collective in the sense that every rank calls them in the same order.
+    ``exchange``: an object with PeerExchange's ``bases``, ``_own_tensor``, ``ensure``, ``barrier`` and ``close`` to use
+    instead of a new PeerExchange (tests run G ranks in one process over shared buffers)."""
 
     MAX_QUERY_ROWS = 131072 + 16384  # two-phase limit + one padded batch
 
-    def __init__(self, dist, group, rank: int, world: int, device: int):
+    def __init__(self, dist, group, rank: int, world: int, device: int, exchange=None):
         import torch
 
         from . import _lib
@@ -149,7 +151,7 @@ class BoundsExchange:
         self.flags_off = 0
         self.slots_off = self.max_batches * world * 4
         nbytes = self.slots_off + self.MAX_QUERY_ROWS * 2 * world * 4
-        self.ex = PeerExchange(dist, group, rank, world, device)
+        self.ex = exchange if exchange is not None else PeerExchange(dist, group, rank, world, device)
         self.ex.ensure(nbytes)
         self.ex._own_tensor.zero_()
         self.ex.barrier()  # nobody pushes into a buffer that is not zeroed yet
@@ -165,23 +167,37 @@ class BoundsExchange:
         self.epoch += 1
         self.n = 2 * rows
 
-    def max_over_ranks(self, b: int, bounds_b) -> None:
-        """bounds_b (2 * rows floats, contiguous) <- element-wise MAX over the ranks, on the current stream."""
+    def _offsets(self, b: int):
+        """Byte offsets of batch b's slots [rank][2 * rows] and flags [rank] in every rank's buffer."""
+        return self.slots_off + b * self.world * self.n * 4, self.flags_off + b * self.world * 4
+
+    def push(self, b: int, bounds_b) -> None:
+        """Stores bounds_b (2 * rows floats, contiguous) into slot [rank] of batch b on every rank, then raises this
+        rank's flag there to the epoch; on the current stream."""
         import ctypes
 
         from .index import _torch_stream
 
-        n, w = self.n, self.world
-        slot_b = self.slots_off + b * w * n * 4
-        flag_b = self.flags_off + b * w * 4
-        slots = (ctypes.c_void_p * w)(*[base + slot_b for base in self.ex.bases])
-        flags = (ctypes.c_void_p * w)(*[base + flag_b for base in self.ex.bases])
-        stream = _torch_stream(self.device)
-        self._check(self._lib.knn_bounds_push_peer_dev(w, self.rank, n, bounds_b.data_ptr(), slots, flags, self.epoch,
-                                                       self.counter.data_ptr(), stream))
+        slot_b, flag_b = self._offsets(b)
+        slots = (ctypes.c_void_p * self.world)(*[base + slot_b for base in self.ex.bases])
+        flags = (ctypes.c_void_p * self.world)(*[base + flag_b for base in self.ex.bases])
+        self._check(self._lib.knn_bounds_push_peer_dev(self.world, self.rank, self.n, bounds_b.data_ptr(), slots, flags,
+                                                       self.epoch, self.counter.data_ptr(), _torch_stream(self.device)))
+
+    def wait_max(self, b: int, bounds_b) -> None:
+        """bounds_b <- element-wise MAX over the slots of batch b in this rank's buffer, once every rank has pushed
+        them; on the current stream."""
+        from .index import _torch_stream
+
+        slot_b, flag_b = self._offsets(b)
         own = self.ex.bases[self.rank]
-        self._check(self._lib.knn_bounds_wait_max_dev(w, n, own + slot_b, own + flag_b, self.epoch, bounds_b.data_ptr(),
-                                                      self.timeout.data_ptr(), stream))
+        self._check(self._lib.knn_bounds_wait_max_dev(self.world, self.n, own + slot_b, own + flag_b, self.epoch,
+                                                      bounds_b.data_ptr(), self.timeout.data_ptr(), _torch_stream(self.device)))
+
+    def max_over_ranks(self, b: int, bounds_b) -> None:
+        """bounds_b (2 * rows floats, contiguous) <- element-wise MAX over the ranks, on the current stream."""
+        self.push(b, bounds_b)
+        self.wait_max(b, bounds_b)
 
     def check(self) -> None:
         if int(self.timeout.item()):
