@@ -46,6 +46,18 @@ extern "C" {
 /* knn_index_create flags */
 #define KNN_FLAG_BF16_STORAGE 1u /* keep only bf16 rows (the bf16 values ARE the database; config C5) */
 
+/* Element type of caller rows (database rows and queries) for the `_typed` entry points.  Protein-language-model
+ * embeddings usually come in 16 bits (ProtT5's half-precision model writes fp16, C5's database is bf16); the typed
+ * calls read them as they are, without an fp32 copy on the host or the device.
+ * Contract: a typed call with fp16 or bf16 rows returns exactly what the same call returns on the rows up-converted to
+ * fp32 (float(x), which is exact): the same D and I bits, the same stored rows (reconstruct) and the same shadow format.
+ * The kernels convert each element at its load and then run the fp32 arithmetic unchanged, and the error bound of the
+ * tensor path is computed from the MEASURED rounding of the up-converted values, never assumed.  D stays float32 and
+ * I int64.  An unknown dtype code returns KNN_ERR_INVALID.  The untyped entry points are the KNN_DTYPE_F32 calls. */
+#define KNN_DTYPE_F32 0  /* float32 */
+#define KNN_DTYPE_F16 1  /* IEEE binary16 */
+#define KNN_DTYPE_BF16 2 /* bfloat16 */
+
 typedef struct knn_index knn_index;
 
 /* Message of the last error on the calling thread ("" if none). */
@@ -73,6 +85,11 @@ int knn_index_reserve(knn_index* idx, int64_t n);
  * Appends n rows; ids are the implicit row numbers 0..ntotal-1. */
 int knn_index_add(knn_index* idx, int64_t n, const float* x);
 int knn_index_add_dev(knn_index* idx, int64_t n, const float* x_dev, void* stream);
+/* The same for rows of element type `dtype` (KNN_DTYPE_*).  The host form stages 64 MiB chunks of the caller's
+ * bytes (twice the rows per chunk for 16-bit rows), so 16-bit rows cross PCIe at half the bytes.  With
+ * KNN_FLAG_BF16_STORAGE bf16 rows are stored as they are; fp16 rows are stored as bf16(float(x)). */
+int knn_index_add_typed(knn_index* idx, int64_t n, const void* x, int dtype);
+int knn_index_add_typed_dev(knn_index* idx, int64_t n, const void* x_dev, int dtype, void* stream);
 
 int64_t knn_index_ntotal(const knn_index* idx);
 int knn_index_d(const knn_index* idx);
@@ -87,6 +104,11 @@ int knn_index_metric(const knn_index* idx);
 int knn_index_search(knn_index* idx, int64_t nq, const float* xq, int64_t k, float* D, int64_t* I);
 int knn_index_search_dev(knn_index* idx, int64_t nq, const float* xq_dev, int64_t k, float* D_dev,
                          int64_t* I_dev, int64_t id_base, void* stream);
+/* The same for queries of element type `dtype` (KNN_DTYPE_*); any query dtype searches any index.  The host form
+ * stages and copies the caller's bytes (pinned caller memory is still DMA'd directly). */
+int knn_index_search_typed(knn_index* idx, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I);
+int knn_index_search_typed_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k, float* D_dev,
+                               int64_t* I_dev, int64_t id_base, void* stream);
 
 /* Two-phase search for a row-sharded database (new; see DESIGN.md section 6).  Phase 1 runs the
  * tensor-core filter over this shard and writes lower_dev[q], a lower bound of the TRUE k-th best score
@@ -102,6 +124,12 @@ int knn_index_search_filter_dev(knn_index* idx, int64_t nq, const float* xq_dev,
                                 float* lower_j_dev, void* stream);
 int knn_index_search_finish_dev(knn_index* idx, int64_t nq, const float* xq_dev, int64_t k, const float* lower_dev,
                                 float* D_dev, int64_t* I_dev, int64_t id_base, void* stream);
+/* Typed forms (queries of element type `dtype`); finish must name the same dtype as filter. */
+int knn_index_search_filter_typed_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k,
+                                      float* lower_dev, int64_t j, float* lower_j_dev, void* stream);
+int knn_index_search_finish_typed_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k,
+                                      const float* lower_dev, float* D_dev, int64_t* I_dev, int64_t id_base,
+                                      void* stream);
 
 /* The same two-phase search batch by batch, so that the caller can overlap the exchange + finish of one query batch
  * with the filter of the next on a second stream (knn_b200/distributed.py does: filter of batch b on the main stream,
@@ -120,6 +148,9 @@ int knn_index_search_finish_dev(knn_index* idx, int64_t nq, const float* xq_dev,
  *   end           after every batch has finished (stream-ordered): repairs overflowed queries, closes the search. */
 int knn_index_search_begin_dev(knn_index* idx, int64_t nq, const float* xq_dev, int64_t k, int64_t* nbatches_out,
                                int64_t* batch_rows_out, void* stream);
+/* begin for queries of element type `dtype` (KNN_DTYPE_*); the batch calls below read them in that type. */
+int knn_index_search_begin_typed_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k,
+                                     int64_t* nbatches_out, int64_t* batch_rows_out, void* stream);
 int knn_index_search_filter_batch_dev(knn_index* idx, int64_t b, int64_t j, float* bounds_dev, void* stream);
 int knn_index_search_finish_batch_dev(knn_index* idx, int64_t b, const float* bounds_dev, float* D_dev, int64_t* I_dev,
                                       int64_t id_base, void* stream);

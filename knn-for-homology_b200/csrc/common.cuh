@@ -129,14 +129,21 @@ typedef uint16_t h16_t;   // raw 16-bit storage of a shadow element
 
 // kernels_basic.cu
 int launch_normalize_l2(float* x, int64_t n, int64_t d, cudaStream_t s);
-// src rows of d floats (stride src_ld) -> zero-padded fp32 master rows (optional), 16-bit shadow rows in format
-// `fmt`, |y|^2 (optional) and the running maxima in *stats.  shadow_is_master: the rounded values ARE the row.
+// Element size of a caller row element of dtype KNN_DTYPE_* (0: unknown dtype).
+inline size_t dtype_size(int dtype) {
+    return dtype == KNN_DTYPE_F32 ? 4 : (dtype == KNN_DTYPE_F16 || dtype == KNN_DTYPE_BF16) ? 2 : 0;
+}
+
+// src rows of d elements of `src_dtype` (KNN_DTYPE_*, stride src_ld elements) -> zero-padded fp32 master rows
+// (optional), 16-bit shadow rows in format `fmt`, |y|^2 (optional) and the running maxima in *stats.  16-bit source
+// rows are converted exactly to fp32 at the load: every output equals that of the up-converted rows, bit for bit.
+// shadow_is_master: the rounded values ARE the row.
 // mbits: explicit mantissa bits kept in a bf16 shadow (7 = all of them; ignored for fp16 and for master rows).
-int launch_ingest(const float* src, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32, h16_t* dst_h16, int fmt,
-                  int mbits, bool shadow_is_master, float* norms2, DbStats* stats, cudaStream_t s);
-// Queries -> zero-padded fp32 (ld = dp) and 16-bit copies, |x|^2 and the score error bound eps
-// (see DESIGN.md "error bound"); rows [nq, nq_pad) of the 16-bit copy are zeroed.
-int launch_prep_queries(const float* xq, int64_t nq, int64_t nq_pad, int d, int dp, float* xq_f32,
+int launch_ingest(const void* src, int src_dtype, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32, h16_t* dst_h16,
+                  int fmt, int mbits, bool shadow_is_master, float* norms2, DbStats* stats, cudaStream_t s);
+// Queries (rows of d elements of `xq_dtype`) -> zero-padded fp32 (ld = dp) and 16-bit copies, |x|^2 and the score
+// error bound eps (see DESIGN.md "error bound"); rows [nq, nq_pad) of the 16-bit copy are zeroed.
+int launch_prep_queries(const void* xq, int xq_dtype, int64_t nq, int64_t nq_pad, int d, int dp, float* xq_f32,
                         h16_t* xq_h16, int fmt, int mbits, float* xnorm2, float* eps, const DbStats* stats,
                         int metric, cudaStream_t s);
 // Exact fp32 scores of queries [0, nqt) (nqt <= kScanMaxQueries... looped inside) against rows
@@ -206,8 +213,9 @@ int launch_kth_lower(FilterState st, const float* eps, int64_t nq, int j, bool n
 // thr <- max(thr, max(lower, -neg_lower2) - eps); neg_lower2 may be null
 int launch_apply_lower(float* thr, const float* eps, const float* lower, const float* neg_lower2, int64_t nq, cudaStream_t s);
 int launch_fill_f32(float* p, int64_t n, float v, cudaStream_t s);
-// Overflow repair: out[i] = xq[idx[i]] (rows of d floats); D[idx[i]] = Dt[i], I[idx[i]] = It[i] (rows of k).
-int launch_gather_rows(const float* xq, int d, const int* idx, int64_t n, float* out, cudaStream_t s);
+// Overflow repair: out[i] = float(xq[idx[i]]) (rows of d elements of xq_dtype, written as fp32);
+// D[idx[i]] = Dt[i], I[idx[i]] = It[i] (rows of k).
+int launch_gather_rows(const void* xq, int xq_dtype, int d, const int* idx, int64_t n, float* out, cudaStream_t s);
 int launch_scatter_results(const float* Dt, const int64_t* It, const int* idx, int64_t n, int k, float* D, int64_t* I,
                            cudaStream_t s);
 

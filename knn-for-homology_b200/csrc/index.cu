@@ -171,6 +171,19 @@ inline void host_copy(void* dst, const void* src, size_t bytes) {
     for (auto& t : th) t.join();
 }
 
+// Row `row` of a caller matrix of d elements of dtype KNN_DTYPE_* (queries and added rows may be fp32, fp16 or bf16).
+inline const void* row_at(const void* base, int64_t row, int d, int dtype) {
+    return static_cast<const char*>(base) + size_t(row) * size_t(d) * dtype_size(dtype);
+}
+
+inline int check_dtype(int dtype, const char* who) {
+    if (dtype_size(dtype) == 0) {
+        set_error("%s: unknown dtype %d (KNN_DTYPE_F32, KNN_DTYPE_F16 or KNN_DTYPE_BF16)", who, dtype);
+        return KNN_ERR_INVALID;
+    }
+    return KNN_OK;
+}
+
 // true when the driver can DMA straight to / from p (cudaHostAlloc / cudaHostRegister memory)
 inline bool host_pointer_is_pinned(const void* p) {
     cudaPointerAttributes a;
@@ -231,7 +244,8 @@ struct knn_index {
         bool active = false, tensor = false;
         int64_t nq = 0, qb = 0, nbatches = 0;
         int k = 0, cap = 0;
-        const float* xq = nullptr;   // the caller's queries (kept alive by the caller until search_end)
+        const void* xq = nullptr;    // the caller's queries (kept alive by the caller until search_end) ...
+        int dtype = KNN_DTYPE_F32;   // ... and their element type
         long long launches0 = 0;
     } pend;
     // parameters
@@ -379,8 +393,8 @@ int query_mbits(const knn_index* ix) {
 int convert_shadow(knn_index* ix, ShadowChoice c, cudaStream_t s) {
     if (ix->ntotal > 0) {
         KNN_CHECK_CUDA(cudaMemsetAsync(ix->stats, 0, sizeof(DbStats), s));
-        KNN_CHECK(launch_ingest(ix->xb_f32, ix->dp, ix->ntotal, ix->dp, ix->dp, nullptr, ix->xb_h16, c.fmt, c.mbits, false,
-                                nullptr, ix->stats, s));
+        KNN_CHECK(launch_ingest(ix->xb_f32, KNN_DTYPE_F32, ix->dp, ix->ntotal, ix->dp, ix->dp, nullptr, ix->xb_h16, c.fmt,
+                                c.mbits, false, nullptr, ix->stats, s));
         ix->st_shadow_conversions++;
     }
     ix->shadow_fmt = c.fmt;
@@ -416,7 +430,7 @@ int prepare_shadow(knn_index* ix, int64_t k, cudaStream_t s) {
 }
 
 // ---- exact path ---------------------------------------------------------------------------
-int search_exact(knn_index* ix, int64_t nq, const float* xq_dev, int k, float* D, int64_t* I, int64_t id_base,
+int search_exact(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k, float* D, int64_t* I, int64_t id_base,
                  cudaStream_t s) {
     const int largest = ix->metric == KNN_METRIC_INNER_PRODUCT;
     const int64_t N = ix->ntotal;
@@ -437,8 +451,8 @@ int search_exact(knn_index* ix, int64_t nq, const float* xq_dev, int k, float* D
     KNN_CHECK(ix->lists_i.ensure(size_t(qb) * list_ld * sizeof(uint32_t)));
     for (int64_t q0 = 0; q0 < nq; q0 += qb) {
         const int64_t nb = nq - q0 < qb ? nq - q0 : qb;
-        KNN_CHECK(launch_prep_queries(xq_dev + q0 * ix->d, nb, nb, ix->d, ix->dp, ix->xq_f32.as<float>(), nullptr, kFmtBF16, 7,
-                                      ix->xnorm2.as<float>(), ix->eps.as<float>(), ix->stats, ix->metric, s));
+        KNN_CHECK(launch_prep_queries(row_at(xq_dev, q0, ix->d, qdt), qdt, nb, nb, ix->d, ix->dp, ix->xq_f32.as<float>(), nullptr,
+                                      kFmtBF16, 7, ix->xnorm2.as<float>(), ix->eps.as<float>(), ix->stats, ix->metric, s));
         for (int64_t j0 = 0; j0 < N; j0 += chunk) {
             const int64_t j1 = j0 + chunk < N ? j0 + chunk : N;
             KNN_CHECK(launch_scan_f32(ix->xq_f32.as<float>(), ix->xnorm2.as<float>(), nb, ix->dp, ix->xb_f32,
@@ -504,7 +518,7 @@ int tensor_prepare(knn_index* ix) {
 // Filter phase of one query batch (rows [off, off+nb) of W): tensor-core scores over database panels of
 // growing size, survivors appended to the candidate lists, thresholds tightened after every panel.
 // On return thr[q] = (k-th best approximate score) - 2 eps[q].
-int tensor_filter_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int64_t nb, const float* xq_batch, int k,
+int tensor_filter_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int64_t nb, const void* xq_batch, int qdt, int k,
                         int cap, int* d_overflow, int* d_ovf_q, cudaStream_t s) {
     const int64_t N = ix->ntotal;
     const int64_t nb_pad = round_up(nb, 256);
@@ -522,8 +536,8 @@ int tensor_filter_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int6
     float* xq_f32 = W.xq_f32.as<float>() + off * ix->dp;
     h16_t* xq_h16 = W.xq_h16.as<h16_t>() + off * ix->dp;
     const int fmt_q = ix->shadow_fmt;  // tcgen05.mma kind::f16 takes one 16-bit format per launch (mixing them is an illegal instruction)
-    KNN_CHECK(launch_prep_queries(xq_batch, nb, nb_pad, ix->d, ix->dp, xq_f32, xq_h16, fmt_q, query_mbits(ix), W.xnorm2.as<float>() + off,
-                                  W.eps.as<float>() + off, ix->stats, ix->metric, s));
+    KNN_CHECK(launch_prep_queries(xq_batch, qdt, nb, nb_pad, ix->d, ix->dp, xq_f32, xq_h16, fmt_q, query_mbits(ix),
+                                  W.xnorm2.as<float>() + off, W.eps.as<float>() + off, ix->stats, ix->metric, s));
     KNN_CHECK(launch_init_filter(st, nb, nb_pad, int(first_panel), s));
     int64_t j0 = 0;
     int panel = 0;
@@ -568,7 +582,7 @@ int tensor_finish_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int6
     return KNN_OK;
 }
 
-int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const float* xq_dev, int k, float* D,
+int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const void* xq_dev, int qdt, int k, float* D,
                     int64_t* I, int64_t id_base, cudaStream_t s) {
     // A candidate list that ran past its capacity (heavily duplicated / clustered scores) is never truncated
     // silently: exactly the queries it happened to are redone with the exact scan and their rows replaced.
@@ -597,8 +611,9 @@ int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, con
         KNN_CHECK(ix->ovf_D.ensure(sizeof(float) * size_t(chunk) * k));
         KNN_CHECK(ix->ovf_I.ensure(sizeof(int64_t) * size_t(chunk) * k));
         KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_idx.p, redo.data() + c0, sizeof(int) * size_t(n), cudaMemcpyHostToDevice, s));
-        KNN_CHECK(launch_gather_rows(xq_dev, ix->d, ix->ovf_idx.as<int>(), n, ix->ovf_x.as<float>(), s));
-        KNN_CHECK(search_exact(ix, n, ix->ovf_x.as<float>(), k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), id_base, s));
+        // the flagged rows are gathered as fp32 (exact for 16-bit queries): the scan sees the values it would have seen
+        KNN_CHECK(launch_gather_rows(xq_dev, qdt, ix->d, ix->ovf_idx.as<int>(), n, ix->ovf_x.as<float>(), s));
+        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, KNN_DTYPE_F32, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), id_base, s));
         KNN_CHECK(launch_scatter_results(ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), ix->ovf_idx.as<int>(), n, k, D, I, s));
         KNN_CHECK_CUDA(cudaStreamSynchronize(s));  // `redo` chunk consumed
     }
@@ -612,7 +627,8 @@ int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, con
 // directly.  Everything is enqueued asynchronously; the host only ever waits for the slot it is about to reuse.
 struct HostPipe {
     knn_index* ix;
-    const float* xq;
+    const void* xq;
+    int qdt;  // element type of xq: the bounce buffers and copies move the caller's bytes as they are
     float* D;
     int64_t* I;
     int k;
@@ -620,7 +636,7 @@ struct HostPipe {
     int64_t slot_q0[2] = {-1, -1}, slot_nb[2] = {0, 0};
 
     int init(int64_t qb) {
-        const size_t in_bytes = size_t(qb) * ix->d * sizeof(float);
+        const size_t in_bytes = size_t(qb) * ix->d * dtype_size(qdt);
         for (int w = 0; w < 2; ++w) {
             KNN_CHECK(ix->hp_xq[w].ensure(in_bytes));
             KNN_CHECK(ix->hp_D[w].ensure(size_t(qb) * k * sizeof(float)));
@@ -647,19 +663,19 @@ struct HostPipe {
     // before batch b: its queries on the way to the device, `s` ordered behind the copy.  The input slot is free as
     // soon as the filter of batch b - 2 has read it - NOT when that batch's results are home: its finish phase runs at
     // low priority under the filter of batch b - 1, and staging the next queries must not wait for it.
-    int acquire(int64_t b, int64_t q0, int64_t nb, cudaStream_t s, const float** xq_b, float** D_b, int64_t** I_b) {
+    int acquire(int64_t b, int64_t q0, int64_t nb, cudaStream_t s, const void** xq_b, float** D_b, int64_t** I_b) {
         const int w = int(b & 1);
         if (b >= 2) KNN_CHECK_CUDA(cudaEventSynchronize(ix->hp_in_free[w]));
-        const size_t bytes = size_t(nb) * ix->d * sizeof(float);
-        const float* src = xq + q0 * ix->d;
+        const size_t bytes = size_t(nb) * ix->d * dtype_size(qdt);
+        const void* src = row_at(xq, q0, ix->d, qdt);
         if (!in_pinned) {
             host_copy(ix->hp_pin_xq[w].p, src, bytes);
-            src = ix->hp_pin_xq[w].as<float>();
+            src = ix->hp_pin_xq[w].p;
         }
         KNN_CHECK_CUDA(cudaMemcpyAsync(ix->hp_xq[w].p, src, bytes, cudaMemcpyHostToDevice, ix->copy_in));
         KNN_CHECK_CUDA(cudaEventRecord(ix->hp_in_ready[w], ix->copy_in));
         KNN_CHECK_CUDA(cudaStreamWaitEvent(s, ix->hp_in_ready[w], 0));
-        *xq_b = ix->hp_xq[w].as<float>();
+        *xq_b = ix->hp_xq[w].p;
         *D_b = ix->hp_D[w].as<float>();
         *I_b = ix->hp_I[w].as<int64_t>();
         return KNN_OK;
@@ -694,8 +710,8 @@ struct HostPipe {
 
 // Overflow repair of a host-pointer search: the flagged queries (rare: heavily duplicated rows, out-of-range data) are
 // uploaded again, answered by the exact scan and written into the caller's rows.
-int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const float* xq, int k, float* D, int64_t* I,
-                         cudaStream_t s) {
+int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const void* xq, int qdt, int k, float* D,
+                         int64_t* I, cudaStream_t s) {
     std::vector<int> h_overflow(size_t(nbatches), 0);
     KNN_CHECK_CUDA(cudaMemcpyAsync(h_overflow.data(), ix->overflow.p, sizeof(int) * size_t(nbatches), cudaMemcpyDeviceToHost, s));
     KNN_CHECK_CUDA(cudaStreamSynchronize(s));
@@ -713,17 +729,19 @@ int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches
     }
     ix->st_overflow_queries += (long long)redo.size();
     const int64_t chunk = 1024;
-    std::vector<float> hx, hD;
+    const size_t row_bytes = size_t(ix->d) * dtype_size(qdt);  // the rows travel in the caller's element type
+    std::vector<char> hx;
+    std::vector<float> hD;
     std::vector<int64_t> hI;
     for (size_t c0 = 0; c0 < redo.size(); c0 += size_t(chunk)) {
         const int64_t n = int64_t(std::min(redo.size() - c0, size_t(chunk)));
-        KNN_CHECK(ix->ovf_x.ensure(sizeof(float) * size_t(chunk) * ix->d));
+        KNN_CHECK(ix->ovf_x.ensure(row_bytes * size_t(chunk)));
         KNN_CHECK(ix->ovf_D.ensure(sizeof(float) * size_t(chunk) * k));
         KNN_CHECK(ix->ovf_I.ensure(sizeof(int64_t) * size_t(chunk) * k));
-        hx.resize(size_t(n) * ix->d);
-        for (int64_t i = 0; i < n; ++i) memcpy(hx.data() + i * ix->d, xq + int64_t(redo[c0 + size_t(i)]) * ix->d, sizeof(float) * ix->d);
-        KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_x.p, hx.data(), sizeof(float) * hx.size(), cudaMemcpyHostToDevice, s));
-        KNN_CHECK(search_exact(ix, n, ix->ovf_x.as<float>(), k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), 0, s));
+        hx.resize(size_t(n) * row_bytes);
+        for (int64_t i = 0; i < n; ++i) memcpy(hx.data() + i * row_bytes, row_at(xq, redo[c0 + size_t(i)], ix->d, qdt), row_bytes);
+        KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_x.p, hx.data(), hx.size(), cudaMemcpyHostToDevice, s));
+        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, qdt, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), 0, s));
         hD.resize(size_t(n) * k);
         hI.resize(size_t(n) * k);
         KNN_CHECK_CUDA(cudaMemcpyAsync(hD.data(), ix->ovf_D.p, sizeof(float) * hD.size(), cudaMemcpyDeviceToHost, s));
@@ -738,7 +756,7 @@ int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches
 }
 
 // `hp` (host-pointer search): xq_dev / D / I are then HOST pointers that only the pipe touches.
-int search_tensor(knn_index* ix, int64_t nq, const float* xq_dev, int k, float* D, int64_t* I, int64_t id_base,
+int search_tensor(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k, float* D, int64_t* I, int64_t id_base,
                   cudaStream_t s, HostPipe* hp = nullptr) {
     const int cap = candidate_capacity(k, ix->ntotal, ix->dense_small_db != 0);
     int64_t qb = ix->query_batch;
@@ -780,12 +798,12 @@ int search_tensor(knn_index* ix, int64_t nq, const float* xq_dev, int k, float* 
         const int64_t q0 = b * qb;
         const int64_t nb = nq - q0 < qb ? nq - q0 : qb;
         const int w = overlap ? int(b & 1) : 0;
-        const float* xq_b = hp ? nullptr : xq_dev + q0 * ix->d;
+        const void* xq_b = hp ? nullptr : row_at(xq_dev, q0, ix->d, qdt);
         float* D_b = hp ? nullptr : D + q0 * k;
         int64_t* I_b = hp ? nullptr : I + q0 * k;
         if (hp) KNN_CHECK(hp->acquire(b, q0, nb, s, &xq_b, &D_b, &I_b));
         if (overlap && b >= 2) KNN_CHECK_CUDA(cudaStreamWaitEvent(s, ix->ev_finished[w], 0));  // ws1[w] is free again
-        KNN_CHECK(tensor_filter_batch(ix, ix->ws1[w], 0, nb, xq_b, k, cap, ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, s));
+        KNN_CHECK(tensor_filter_batch(ix, ix->ws1[w], 0, nb, xq_b, qdt, k, cap, ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, s));
         if (hp) {
             KNN_CHECK(hp->filtered(b, s));
             KNN_CHECK(hp->before_finish(b));
@@ -809,9 +827,9 @@ int search_tensor(knn_index* ix, int64_t nq, const float* xq_dev, int k, float* 
     }
     if (hp) {
         KNN_CHECK(hp->finish());
-        return redo_overflowed_host(ix, nq, qb, nbatches, xq_dev, k, D, I, s);
+        return redo_overflowed_host(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, s);
     }
-    return redo_overflowed(ix, nq, qb, nbatches, xq_dev, k, D, I, id_base, s);
+    return redo_overflowed(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, id_base, s);
 }
 
 bool use_tensor_path(const knn_index* ix, int64_t nq, int k) {
@@ -820,12 +838,13 @@ bool use_tensor_path(const knn_index* ix, int64_t nq, int k) {
     return tensor;
 }
 
-int search_dev_impl(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, float* D, int64_t* I, int64_t id_base,
+int search_dev_impl(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int64_t k64, float* D, int64_t* I, int64_t id_base,
                     cudaStream_t s, HostPipe* hp = nullptr) {
     if (nq < 0 || k64 <= 0 || (nq > 0 && (!xq_dev || !D || !I))) {
         set_error("search: invalid arguments (nq=%lld, k=%lld)", (long long)nq, (long long)k64);
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(qdt, "search"));
     if (k64 > KNN_MAX_K) {
         set_error("search: k=%lld exceeds KNN_MAX_K=%d", (long long)k64, KNN_MAX_K);
         return KNN_ERR_LIMIT;
@@ -857,7 +876,8 @@ int search_dev_impl(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64,
             set_error("internal: host pipe on the exact path");
             return KNN_ERR_INVALID;
         }
-        rc = tensor ? search_tensor(ix, nq, xq_dev, k, D, I, id_base, s, hp) : search_exact(ix, nq, xq_dev, k, D, I, id_base, s);
+        rc = tensor ? search_tensor(ix, nq, xq_dev, qdt, k, D, I, id_base, s, hp)
+                    : search_exact(ix, nq, xq_dev, qdt, k, D, I, id_base, s);
     }
     if (rc != KNN_OK) return rc;
     KNN_CHECK_CUDA(cudaEventRecord(ix->search_event, s));
@@ -1045,11 +1065,12 @@ int knn_index_reserve(knn_index* ix, int64_t n) {
     return grow(ix, n, /*exact=*/true);
 }
 
-int knn_index_add_dev(knn_index* ix, int64_t n, const float* x_dev, void* stream) {
+int knn_index_add_typed_dev(knn_index* ix, int64_t n, const void* x_dev, int dtype, void* stream) {
     if (!ix || n < 0 || (n > 0 && !x_dev)) {
         set_error("add: invalid arguments");
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(dtype, "add"));
     if (n == 0) return KNN_OK;
     DeviceGuard g(ix->device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -1062,7 +1083,7 @@ int knn_index_add_dev(knn_index* ix, int64_t n, const float* x_dev, void* stream
         ix->shadow_fmt = c.fmt;
         ix->shadow_mbits = c.mbits;
     }
-    KNN_CHECK(launch_ingest(x_dev, ix->d, n, ix->d, ix->dp, ix->xb_f32 ? ix->xb_f32 + r0 * ix->dp : nullptr,
+    KNN_CHECK(launch_ingest(x_dev, dtype, ix->d, n, ix->d, ix->dp, ix->xb_f32 ? ix->xb_f32 + r0 * ix->dp : nullptr,
                             ix->xb_h16 + r0 * ix->dp, ix->shadow_fmt, ix->shadow_mbits, bf16_only(ix), ix->ynorm2 + r0,
                             ix->stats, s));
     KNN_CHECK_CUDA(cudaEventRecord(ix->add_event, s));
@@ -1071,18 +1092,25 @@ int knn_index_add_dev(knn_index* ix, int64_t n, const float* x_dev, void* stream
     return KNN_OK;
 }
 
-int knn_index_add(knn_index* ix, int64_t n, const float* x) {
+int knn_index_add_dev(knn_index* ix, int64_t n, const float* x_dev, void* stream) {
+    return knn_index_add_typed_dev(ix, n, x_dev, KNN_DTYPE_F32, stream);
+}
+
+int knn_index_add_typed(knn_index* ix, int64_t n, const void* x, int dtype) {
     if (!ix || n < 0 || (n > 0 && !x)) {
         set_error("add: invalid arguments");
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(dtype, "add"));
     if (n == 0) return KNN_OK;
     DeviceGuard g(ix->device);
     KNN_CHECK(grow(ix, ix->ntotal + n));
     // chunks of <= 64 MiB through two staging buffers: the H2D copy of chunk i + 1 (copy stream) runs while chunk i is
-    // ingested (index stream); pageable caller memory goes through the driver's own bounce buffers
-    const int64_t rows_per = std::max<int64_t>(1, (int64_t(64) << 20) / (int64_t(ix->d) * 4));
-    const size_t stage_bytes = size_t(n < rows_per ? n : rows_per) * ix->d * sizeof(float);
+    // ingested (index stream); pageable caller memory goes through the driver's own bounce buffers.  The chunks hold the
+    // caller's bytes as they are: 16-bit rows are converted by the ingest kernel, not before the copy.
+    const size_t row_bytes = size_t(ix->d) * dtype_size(dtype);
+    const int64_t rows_per = std::max<int64_t>(1, (int64_t(64) << 20) / int64_t(row_bytes));
+    const size_t stage_bytes = size_t(n < rows_per ? n : rows_per) * row_bytes;
     KNN_CHECK(ix->stage.ensure(stage_bytes));
     if (n > rows_per) KNN_CHECK(ix->stage2.ensure(stage_bytes));
     int64_t c = 0;
@@ -1090,12 +1118,12 @@ int knn_index_add(knn_index* ix, int64_t n, const float* x) {
         for (int64_t r0 = 0; r0 < n; r0 += rows_per, ++c) {
             const int64_t nr = n - r0 < rows_per ? n - r0 : rows_per;
             const int w = int(c & 1);
-            float* st = (w ? ix->stage2 : ix->stage).as<float>();
+            void* st = (w ? ix->stage2 : ix->stage).p;
             if (c >= 2) KNN_CHECK_CUDA(cudaEventSynchronize(ix->stage_free[w]));  // the ingest that read this buffer is done
-            KNN_CHECK_CUDA(cudaMemcpyAsync(st, x + r0 * ix->d, size_t(nr) * ix->d * sizeof(float), cudaMemcpyHostToDevice, ix->copy_in));
+            KNN_CHECK_CUDA(cudaMemcpyAsync(st, row_at(x, r0, ix->d, dtype), size_t(nr) * row_bytes, cudaMemcpyHostToDevice, ix->copy_in));
             KNN_CHECK_CUDA(cudaEventRecord(ix->hp_in_ready[w], ix->copy_in));
             KNN_CHECK_CUDA(cudaStreamWaitEvent(ix->stream, ix->hp_in_ready[w], 0));
-            KNN_CHECK(knn_index_add_dev(ix, nr, st, ix->stream));
+            KNN_CHECK(knn_index_add_typed_dev(ix, nr, st, dtype, ix->stream));
             KNN_CHECK_CUDA(cudaEventRecord(ix->stage_free[w], ix->stream));
         }
         return KNN_OK;
@@ -1110,25 +1138,33 @@ int knn_index_add(knn_index* ix, int64_t n, const float* x) {
     return KNN_OK;
 }
 
+int knn_index_add(knn_index* ix, int64_t n, const float* x) { return knn_index_add_typed(ix, n, x, KNN_DTYPE_F32); }
+
 int64_t knn_index_ntotal(const knn_index* ix) { return ix ? ix->ntotal : -1; }
 int knn_index_d(const knn_index* ix) { return ix ? ix->d : -1; }
 int knn_index_metric(const knn_index* ix) { return ix ? ix->metric : -1; }
 
-int knn_index_search_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k, float* D_dev, int64_t* I_dev,
-                         int64_t id_base, void* stream) {
+int knn_index_search_typed_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k, float* D_dev,
+                               int64_t* I_dev, int64_t id_base, void* stream) {
     if (!ix) {
         set_error("search: null index");
         return KNN_ERR_INVALID;
     }
     DeviceGuard g(ix->device);
-    return search_dev_impl(ix, nq, xq_dev, k, D_dev, I_dev, id_base, static_cast<cudaStream_t>(stream));
+    return search_dev_impl(ix, nq, xq_dev, dtype, k, D_dev, I_dev, id_base, static_cast<cudaStream_t>(stream));
 }
 
-int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, float* D, int64_t* I) {
+int knn_index_search_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k, float* D_dev, int64_t* I_dev,
+                         int64_t id_base, void* stream) {
+    return knn_index_search_typed_dev(ix, nq, xq_dev, KNN_DTYPE_F32, k, D_dev, I_dev, id_base, stream);
+}
+
+int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I) {
     if (!ix || nq < 0 || k <= 0 || (nq > 0 && (!xq || !D || !I))) {
         set_error("search: invalid arguments (nq=%lld, k=%lld)", (long long)nq, (long long)k);
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(dtype, "search"));
     if (k > KNN_MAX_K) {
         set_error("search: k=%lld exceeds KNN_MAX_K=%d", (long long)k, KNN_MAX_K);
         return KNN_ERR_LIMIT;
@@ -1137,8 +1173,8 @@ int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, floa
     DeviceGuard g(ix->device);
     if (ix->ntotal > 0 && use_tensor_path(ix, nq, int(k))) {
         // tensor path: one pipelined pass over the query batches (copies under compute, see HostPipe)
-        HostPipe hp{ix, xq, D, I, int(k), host_pointer_is_pinned(xq), host_pointer_is_pinned(D) && host_pointer_is_pinned(I)};
-        const int rc = search_dev_impl(ix, nq, xq, k, D, I, 0, ix->stream, &hp);
+        HostPipe hp{ix, xq, dtype, D, I, int(k), host_pointer_is_pinned(xq), host_pointer_is_pinned(D) && host_pointer_is_pinned(I)};
+        const int rc = search_dev_impl(ix, nq, xq, dtype, k, D, I, 0, ix->stream, &hp);
         if (rc != KNN_OK) {
             // copies into / out of the caller's arrays may still be in flight on the copy streams: nothing may touch
             // the caller's memory once this call has returned, error or not
@@ -1152,15 +1188,16 @@ int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, floa
     // H2D -> search -> D2H on one stream
     const int64_t hb = 65536;
     const int64_t nb_max = nq < hb ? nq : hb;
-    KNN_CHECK(ix->h_xq.ensure(size_t(nb_max) * ix->d * sizeof(float)));
+    const size_t row_bytes = size_t(ix->d) * dtype_size(dtype);  // queries are staged in the caller's element type
+    KNN_CHECK(ix->h_xq.ensure(size_t(nb_max) * row_bytes));
     KNN_CHECK(ix->h_D.ensure(size_t(nb_max) * k * sizeof(float)));
     KNN_CHECK(ix->h_I.ensure(size_t(nb_max) * k * sizeof(int64_t)));
     long long launches = 0, gemm_launches = 0, overflow = 0, overflow_q = 0;
     double gemm_ms = 0;
     for (int64_t q0 = 0; q0 < nq; q0 += hb) {
         const int64_t nb = nq - q0 < hb ? nq - q0 : hb;
-        KNN_CHECK_CUDA(cudaMemcpyAsync(ix->h_xq.p, xq + q0 * ix->d, size_t(nb) * ix->d * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-        KNN_CHECK(search_dev_impl(ix, nb, ix->h_xq.as<float>(), k, ix->h_D.as<float>(), ix->h_I.as<int64_t>(), 0, ix->stream));
+        KNN_CHECK_CUDA(cudaMemcpyAsync(ix->h_xq.p, row_at(xq, q0, ix->d, dtype), size_t(nb) * row_bytes, cudaMemcpyHostToDevice, ix->stream));
+        KNN_CHECK(search_dev_impl(ix, nb, ix->h_xq.p, dtype, k, ix->h_D.as<float>(), ix->h_I.as<int64_t>(), 0, ix->stream));
         KNN_CHECK_CUDA(cudaMemcpyAsync(D + q0 * k, ix->h_D.p, size_t(nb) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
         KNN_CHECK_CUDA(cudaMemcpyAsync(I + q0 * k, ix->h_I.p, size_t(nb) * k * sizeof(int64_t), cudaMemcpyDeviceToHost, ix->stream));
         KNN_CHECK_CUDA(cudaStreamSynchronize(ix->stream));
@@ -1178,15 +1215,20 @@ int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, floa
     return KNN_OK;
 }
 
+int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, float* D, int64_t* I) {
+    return knn_index_search_typed(ix, nq, xq, KNN_DTYPE_F32, k, D, I);
+}
+
 // ---- two-phase (row-sharded) search ---------------------------------------------------------
 // begin -> per batch: filter_batch ... (caller combines the bounds of all shards) ... finish_batch -> end.
 // The batch-wise calls let the caller run exchange + finish of batch b on another stream under the filter of batch
 // b + 1 (knn_b200/distributed.py); knn_index_search_filter_dev / _finish_dev are the all-batches-at-once form.
-static int two_phase_begin(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, cudaStream_t s, const char* who) {
+static int two_phase_begin(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int64_t k64, cudaStream_t s, const char* who) {
     if (!ix || nq <= 0 || k64 <= 0 || !xq_dev) {
         set_error("%s: invalid arguments", who);
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(qdt, who));
     if (k64 > KNN_MAX_K) {
         set_error("%s: k=%lld exceeds KNN_MAX_K=%d", who, (long long)k64, KNN_MAX_K);
         return KNN_ERR_LIMIT;
@@ -1209,6 +1251,7 @@ static int two_phase_begin(knn_index* ix, int64_t nq, const float* xq_dev, int64
     P.nq = nq;
     P.k = k;
     P.xq = xq_dev;
+    P.dtype = qdt;
     P.launches0 = g_launches.load();
     P.tensor = ix->ntotal > 0 && use_tensor_path(ix, nq, k);
     ix->last_path = P.tensor ? 2 : 1;
@@ -1250,8 +1293,8 @@ static int two_phase_filter_batch(knn_index* ix, int64_t b, float* lower_b, int6
         if (lower_j_b) KNN_CHECK(launch_fill_f32(lower_j_b, nb, negate_j ? FLT_MAX : -FLT_MAX, s));
         return KNN_OK;
     }
-    KNN_CHECK(tensor_filter_batch(ix, ix->ws2, q0, nb, P.xq + q0 * ix->d, P.k, P.cap, ix->overflow.as<int>() + b,
-                                  ix->ovf_q.as<int>() + q0, s));
+    KNN_CHECK(tensor_filter_batch(ix, ix->ws2, q0, nb, row_at(P.xq, q0, ix->d, P.dtype), P.dtype, P.k, P.cap,
+                                  ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, s));
     KNN_CHECK(launch_export_lower(ix->ws2.thr.as<float>() + q0, ix->ws2.eps.as<float>() + q0, nb, lower_b, s));
     if (lower_j_b) {
         KNN_CHECK(launch_kth_lower(filter_state(ix->ws2, q0, P.cap), ix->ws2.eps.as<float>() + q0, nb, int(j), negate_j, lower_j_b, s));
@@ -1269,7 +1312,8 @@ static int two_phase_finish_batch(knn_index* ix, int64_t b, const float* lower_b
         // path whenever all of them do.  The scan uses the index's shared scratch (xq_f32, scores, lists): every batch of
         // an exact shard must be finished on the same stream.
         const long long l0 = P.launches0;
-        KNN_CHECK(search_dev_impl(ix, nb, P.xq + q0 * ix->d, P.k, D_dev + q0 * P.k, I_dev + q0 * P.k, id_base, s));
+        KNN_CHECK(search_dev_impl(ix, nb, row_at(P.xq, q0, ix->d, P.dtype), P.dtype, P.k, D_dev + q0 * P.k, I_dev + q0 * P.k,
+                                  id_base, s));
         P.launches0 = l0;
         return KNN_OK;
     }
@@ -1279,7 +1323,7 @@ static int two_phase_finish_batch(knn_index* ix, int64_t b, const float* lower_b
 static int two_phase_end(knn_index* ix, float* D_dev, int64_t* I_dev, int64_t id_base, cudaStream_t s) {
     auto& P = ix->pend;
     P.active = false;
-    if (P.tensor) KNN_CHECK(redo_overflowed(ix, P.nq, P.qb, P.nbatches, P.xq, P.k, D_dev, I_dev, id_base, s));
+    if (P.tensor) KNN_CHECK(redo_overflowed(ix, P.nq, P.qb, P.nbatches, P.xq, P.dtype, P.k, D_dev, I_dev, id_base, s));
     KNN_CHECK_CUDA(cudaEventRecord(ix->search_event, s));
     if (ix->profile && ix->ev_used) {
         KNN_CHECK_CUDA(cudaStreamSynchronize(s));
@@ -1289,17 +1333,22 @@ static int two_phase_end(knn_index* ix, float* D_dev, int64_t* I_dev, int64_t id
     return KNN_OK;
 }
 
-int knn_index_search_begin_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k, int64_t* nbatches_out,
-                               int64_t* batch_rows_out, void* stream) {
+int knn_index_search_begin_typed_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k,
+                                     int64_t* nbatches_out, int64_t* batch_rows_out, void* stream) {
     if (!ix || !nbatches_out || !batch_rows_out) {
         set_error("search_begin: invalid arguments");
         return KNN_ERR_INVALID;
     }
     DeviceGuard g(ix->device);
-    KNN_CHECK(two_phase_begin(ix, nq, xq_dev, k, static_cast<cudaStream_t>(stream), "search_begin"));
+    KNN_CHECK(two_phase_begin(ix, nq, xq_dev, dtype, k, static_cast<cudaStream_t>(stream), "search_begin"));
     *nbatches_out = ix->pend.nbatches;
     *batch_rows_out = ix->pend.qb;
     return KNN_OK;
+}
+
+int knn_index_search_begin_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k, int64_t* nbatches_out,
+                               int64_t* batch_rows_out, void* stream) {
+    return knn_index_search_begin_typed_dev(ix, nq, xq_dev, KNN_DTYPE_F32, k, nbatches_out, batch_rows_out, stream);
 }
 
 int knn_index_search_filter_batch_dev(knn_index* ix, int64_t b, int64_t j, float* bounds_dev, void* stream) {
@@ -1332,15 +1381,15 @@ int knn_index_search_end_dev(knn_index* ix, float* D_dev, int64_t* I_dev, int64_
     return two_phase_end(ix, D_dev, I_dev, id_base, static_cast<cudaStream_t>(stream));
 }
 
-int knn_index_search_filter_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, float* lower_dev, int64_t j,
-                                float* lower_j_dev, void* stream) {
+int knn_index_search_filter_typed_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k64, float* lower_dev,
+                                      int64_t j, float* lower_j_dev, void* stream) {
     if (!ix || !lower_dev) {
         set_error("search_filter: invalid arguments");
         return KNN_ERR_INVALID;
     }
     DeviceGuard g(ix->device);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    KNN_CHECK(two_phase_begin(ix, nq, xq_dev, k64, s, "search_filter"));
+    KNN_CHECK(two_phase_begin(ix, nq, xq_dev, dtype, k64, s, "search_filter"));
     auto& P = ix->pend;
     for (int64_t b = 0; b < P.nbatches; ++b) {
         const int64_t q0 = b * P.qb;
@@ -1353,14 +1402,20 @@ int knn_index_search_filter_dev(knn_index* ix, int64_t nq, const float* xq_dev, 
     return KNN_OK;
 }
 
-int knn_index_search_finish_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, const float* lower_dev,
-                                float* D_dev, int64_t* I_dev, int64_t id_base, void* stream) {
+int knn_index_search_filter_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, float* lower_dev, int64_t j,
+                                float* lower_j_dev, void* stream) {
+    return knn_index_search_filter_typed_dev(ix, nq, xq_dev, KNN_DTYPE_F32, k64, lower_dev, j, lower_j_dev, stream);
+}
+
+int knn_index_search_finish_typed_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k64,
+                                      const float* lower_dev, float* D_dev, int64_t* I_dev, int64_t id_base, void* stream) {
     if (!ix || !xq_dev || !D_dev || !I_dev) {
         set_error("search_finish: invalid arguments");
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_dtype(dtype, "search_finish"));
     auto& P = ix->pend;
-    if (!P.active || P.nq != nq || P.k != int(k64) || P.xq != xq_dev) {
+    if (!P.active || P.nq != nq || P.k != int(k64) || P.xq != xq_dev || P.dtype != dtype) {
         set_error("search_finish: no matching search_filter call is pending");
         return KNN_ERR_INVALID;
     }
@@ -1374,6 +1429,11 @@ int knn_index_search_finish_dev(knn_index* ix, int64_t nq, const float* xq_dev, 
         }
     }
     return two_phase_end(ix, D_dev, I_dev, id_base, s);
+}
+
+int knn_index_search_finish_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t k64, const float* lower_dev,
+                                float* D_dev, int64_t* I_dev, int64_t id_base, void* stream) {
+    return knn_index_search_finish_typed_dev(ix, nq, xq_dev, KNN_DTYPE_F32, k64, lower_dev, D_dev, I_dev, id_base, stream);
 }
 
 int knn_index_reconstruct(knn_index* ix, int64_t i0, int64_t n, float* out) {

@@ -105,10 +105,31 @@ __device__ __forceinline__ uint32_t pack_shadow2(float a, float b, int mbits, fl
     }
 }
 
+// Elements 4c .. 4c+3 of a caller row, converted to fp32 at the load.  fp16 -> fp32 and bf16 -> fp32 are exact, so
+// everything downstream of the load sees exactly the values of the up-converted row.  16-bit sources load 8 bytes per
+// 4 elements (a uint2, as RowChunk<true> below); the caller guarantees 16-byte (fp32) / 8-byte (16-bit) alignment.
+__device__ __forceinline__ float4 load4_f32(const float* r, int c) { return reinterpret_cast<const float4*>(r)[c]; }
+__device__ __forceinline__ float4 load4_f32(const __half* r, int c) {
+    uint2 p = reinterpret_cast<const uint2*>(r)[c];
+    const float2 a = __half22float2(*reinterpret_cast<__half2*>(&p.x));
+    const float2 b = __half22float2(*reinterpret_cast<__half2*>(&p.y));
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 load4_f32(const __nv_bfloat16* r, int c) {
+    const uint2 p = reinterpret_cast<const uint2*>(r)[c];  // bf16 -> fp32 is a 16-bit shift
+    return make_float4(__uint_as_float(p.x << 16), __uint_as_float(p.x & 0xFFFF0000u), __uint_as_float(p.y << 16),
+                       __uint_as_float(p.y & 0xFFFF0000u));
+}
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+
 // One warp per row.  Writes the zero-padded fp32 master row (optional), the 16-bit shadow row,
 // |y|^2 and folds max|y|^2, max|y - shadow(y)|^2 into *stats (optional).
-template <int FMT>
-__global__ void __launch_bounds__(kBlock) ingest_rows_kernel(const float* __restrict__ src, int64_t src_ld, int64_t n,
+// SRC: element type of the caller's rows (float, __half or __nv_bfloat16); 16-bit rows run the fp32 arithmetic on
+// their exact fp32 values, so every output is bit-identical to ingesting the up-converted rows.
+template <int FMT, class SRC>
+__global__ void __launch_bounds__(kBlock) ingest_rows_kernel(const SRC* __restrict__ src, int64_t src_ld, int64_t n,
                                                               int d, int dp, float* __restrict__ dst_f32,
                                                               h16_t* __restrict__ dst_h16,
                                                               float* __restrict__ norms2,
@@ -118,18 +139,18 @@ __global__ void __launch_bounds__(kBlock) ingest_rows_kernel(const float* __rest
     const int64_t warps = int64_t(gridDim.x) * kWarpsPerBlock;
     float wmax_n = 0.f, wmax_d = 0.f;
     for (int64_t row = int64_t(blockIdx.x) * kWarpsPerBlock + (threadIdx.x >> 5); row < n; row += warps) {
-        const float* r = src + row * src_ld;
+        const SRC* r = src + row * src_ld;
         float s = 0.f, e = 0.f;
         for (int c = lane; c < dp / 4; c += 32) {
             float4 v;
             const int c0 = c * 4;
             if (vec_ok && c0 + 3 < d) {
-                v = reinterpret_cast<const float4*>(r)[c];
+                v = load4_f32(r, c);
             } else {
-                v.x = c0 + 0 < d ? r[c0 + 0] : 0.f;
-                v.y = c0 + 1 < d ? r[c0 + 1] : 0.f;
-                v.z = c0 + 2 < d ? r[c0 + 2] : 0.f;
-                v.w = c0 + 3 < d ? r[c0 + 3] : 0.f;
+                v.x = c0 + 0 < d ? to_f32(r[c0 + 0]) : 0.f;
+                v.y = c0 + 1 < d ? to_f32(r[c0 + 1]) : 0.f;
+                v.z = c0 + 2 < d ? to_f32(r[c0 + 2]) : 0.f;
+                v.w = c0 + 3 < d ? to_f32(r[c0 + 3]) : 0.f;
             }
             float2 flo, fhi;
             uint2 packed;
@@ -425,33 +446,65 @@ int launch_normalize_l2(float* x, int64_t n, int64_t d, cudaStream_t s) {
     return KNN_OK;
 }
 
-int launch_ingest(const float* src, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32, h16_t* dst_h16, int fmt,
-                  int mbits, bool shadow_is_master, float* norms2, DbStats* stats, cudaStream_t s) {
-    if (n <= 0) return KNN_OK;
-    const int vec_ok = (d % 4 == 0) && (src_ld % 4 == 0) && (reinterpret_cast<uintptr_t>(src) % 16 == 0);
-    const int grid = grid_for_rows(n, kWarpsPerBlock, 8);
+// The vector loads need d % 4 == 0, a row stride that keeps every row aligned and an aligned base pointer: 16 bytes
+// for fp32 rows, 8 bytes for 16-bit rows.  Anything else takes the scalar loads.
+static int vec_loads_ok(const void* src, int64_t src_ld, int d, int src_dtype) {
+    const uintptr_t align = src_dtype == KNN_DTYPE_F32 ? 16 : 8;
+    return (d % 4 == 0) && (src_ld % 4 == 0) && (reinterpret_cast<uintptr_t>(src) % align == 0);
+}
+
+template <class SRC>
+static void ingest_launch_t(int grid, const void* src, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32,
+                            h16_t* dst_h16, int fmt, float* norms2, float* dnorms2, DbStats* stats, int vec_ok,
+                            int shadow_is_master, int mbits, cudaStream_t s) {
+    const SRC* x = static_cast<const SRC*>(src);
     if (fmt == kFmtFP16)
-        ingest_rows_kernel<kFmtFP16><<<grid, kBlock, 0, s>>>(src, src_ld, n, d, dp, dst_f32, dst_h16, norms2, nullptr, stats,
-                                                            vec_ok, shadow_is_master, mbits);
+        ingest_rows_kernel<kFmtFP16, SRC><<<grid, kBlock, 0, s>>>(x, src_ld, n, d, dp, dst_f32, dst_h16, norms2, dnorms2,
+                                                                  stats, vec_ok, shadow_is_master, mbits);
     else
-        ingest_rows_kernel<kFmtBF16><<<grid, kBlock, 0, s>>>(src, src_ld, n, d, dp, dst_f32, dst_h16, norms2, nullptr, stats,
-                                                            vec_ok, shadow_is_master, mbits);
+        ingest_rows_kernel<kFmtBF16, SRC><<<grid, kBlock, 0, s>>>(x, src_ld, n, d, dp, dst_f32, dst_h16, norms2, dnorms2,
+                                                                  stats, vec_ok, shadow_is_master, mbits);
+}
+
+static int ingest_launch(const void* src, int src_dtype, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32,
+                         h16_t* dst_h16, int fmt, float* norms2, float* dnorms2, DbStats* stats, int shadow_is_master,
+                         int mbits, cudaStream_t s) {
+    const int vec_ok = vec_loads_ok(src, src_ld, d, src_dtype);
+    const int grid = grid_for_rows(n, kWarpsPerBlock, 8);
+    switch (src_dtype) {
+        case KNN_DTYPE_F32:
+            ingest_launch_t<float>(grid, src, src_ld, n, d, dp, dst_f32, dst_h16, fmt, norms2, dnorms2, stats, vec_ok,
+                                   shadow_is_master, mbits, s);
+            break;
+        case KNN_DTYPE_F16:
+            ingest_launch_t<__half>(grid, src, src_ld, n, d, dp, dst_f32, dst_h16, fmt, norms2, dnorms2, stats, vec_ok,
+                                    shadow_is_master, mbits, s);
+            break;
+        case KNN_DTYPE_BF16:
+            ingest_launch_t<__nv_bfloat16>(grid, src, src_ld, n, d, dp, dst_f32, dst_h16, fmt, norms2, dnorms2, stats,
+                                           vec_ok, shadow_is_master, mbits, s);
+            break;
+        default:
+            set_error("unknown source dtype %d", src_dtype);
+            return KNN_ERR_INVALID;
+    }
     KNN_CHECK_LAUNCH();
     return KNN_OK;
 }
 
-int launch_prep_queries(const float* xq, int64_t nq, int64_t nq_pad, int d, int dp, float* xq_f32,
+int launch_ingest(const void* src, int src_dtype, int64_t src_ld, int64_t n, int d, int dp, float* dst_f32, h16_t* dst_h16,
+                  int fmt, int mbits, bool shadow_is_master, float* norms2, DbStats* stats, cudaStream_t s) {
+    if (n <= 0) return KNN_OK;
+    return ingest_launch(src, src_dtype, src_ld, n, d, dp, dst_f32, dst_h16, fmt, norms2, nullptr, stats,
+                         shadow_is_master, mbits, s);
+}
+
+int launch_prep_queries(const void* xq, int xq_dtype, int64_t nq, int64_t nq_pad, int d, int dp, float* xq_f32,
                         h16_t* xq_h16, int fmt, int mbits, float* xnorm2, float* eps, const DbStats* stats, int metric,
                         cudaStream_t s) {
     if (nq <= 0) return KNN_OK;
     // eps doubles as scratch for |dx|^2 until query_eps_kernel overwrites it
-    const int vec_ok = (d % 4 == 0) && (reinterpret_cast<uintptr_t>(xq) % 16 == 0);
-    const int grid = grid_for_rows(nq, kWarpsPerBlock, 8);
-    if (fmt == kFmtFP16)
-        ingest_rows_kernel<kFmtFP16><<<grid, kBlock, 0, s>>>(xq, d, nq, d, dp, xq_f32, xq_h16, xnorm2, eps, nullptr, vec_ok, 0, mbits);
-    else
-        ingest_rows_kernel<kFmtBF16><<<grid, kBlock, 0, s>>>(xq, d, nq, d, dp, xq_f32, xq_h16, xnorm2, eps, nullptr, vec_ok, 0, mbits);
-    KNN_CHECK_LAUNCH();
+    KNN_CHECK(ingest_launch(xq, xq_dtype, d, nq, d, dp, xq_f32, xq_h16, fmt, xnorm2, eps, nullptr, 0, mbits, s));
     if (xq_h16 && nq_pad > nq) {
         KNN_CHECK_CUDA(cudaMemsetAsync(xq_h16 + nq * int64_t(dp), 0, size_t(nq_pad - nq) * dp * sizeof(h16_t), s));
     }

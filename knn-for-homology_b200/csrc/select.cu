@@ -622,10 +622,16 @@ __global__ void init_filter_kernel(float* thr, int* counts, int* ovf, int64_t nq
     if (q < nq) ovf[q] = 0;
 }
 
-__global__ void gather_rows_kernel(const float* __restrict__ xq, int d, const int* __restrict__ idx, float* __restrict__ out) {
-    const float* src = xq + int64_t(idx[blockIdx.x]) * d;
+// SRC: element type of the query rows (float, __half, __nv_bfloat16); the fp32 rows written are exact up-conversions.
+__device__ __forceinline__ float elem_f32(float v) { return v; }
+__device__ __forceinline__ float elem_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float elem_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+template <class SRC>
+__global__ void gather_rows_kernel(const SRC* __restrict__ xq, int d, const int* __restrict__ idx, float* __restrict__ out) {
+    const SRC* src = xq + int64_t(idx[blockIdx.x]) * d;
     float* dst = out + int64_t(blockIdx.x) * d;
-    for (int i = threadIdx.x; i < d; i += blockDim.x) dst[i] = src[i];
+    for (int i = threadIdx.x; i < d; i += blockDim.x) dst[i] = elem_f32(src[i]);
 }
 
 __global__ void scatter_results_kernel(const float* __restrict__ Dt, const int64_t* __restrict__ It, const int* __restrict__ idx,
@@ -726,9 +732,18 @@ int launch_init_filter(FilterState st, int64_t nq, int64_t nq_pad, int first_cou
     return KNN_OK;
 }
 
-int launch_gather_rows(const float* xq, int d, const int* idx, int64_t n, float* out, cudaStream_t s) {
+int launch_gather_rows(const void* xq, int xq_dtype, int d, const int* idx, int64_t n, float* out, cudaStream_t s) {
     if (n <= 0) return KNN_OK;
-    gather_rows_kernel<<<unsigned(n), 256, 0, s>>>(xq, d, idx, out);
+    switch (xq_dtype) {
+        case KNN_DTYPE_F32: gather_rows_kernel<<<unsigned(n), 256, 0, s>>>(static_cast<const float*>(xq), d, idx, out); break;
+        case KNN_DTYPE_F16: gather_rows_kernel<<<unsigned(n), 256, 0, s>>>(static_cast<const __half*>(xq), d, idx, out); break;
+        case KNN_DTYPE_BF16:
+            gather_rows_kernel<<<unsigned(n), 256, 0, s>>>(static_cast<const __nv_bfloat16*>(xq), d, idx, out);
+            break;
+        default:
+            set_error("unknown query dtype %d", xq_dtype);
+            return KNN_ERR_INVALID;
+    }
     KNN_CHECK_LAUNCH();
     return KNN_OK;
 }

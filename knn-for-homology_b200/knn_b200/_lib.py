@@ -16,6 +16,11 @@ LIB_PATH = Path(os.environ.get("KNN_B200_LIB", _HERE.parent / "libknn_b200.so"))
 c_i64 = ctypes.c_int64
 c_vp = ctypes.c_void_p
 
+# element types of caller rows for the *_typed entry points (KNN_DTYPE_* in include/knn_b200.h)
+DTYPE_F32 = 0
+DTYPE_F16 = 1
+DTYPE_BF16 = 2
+
 # name -> (restype, argtypes); mirrors include/knn_b200.h one to one
 SIGNATURES = {
     "knn_last_error": (ctypes.c_char_p, []),
@@ -40,6 +45,15 @@ SIGNATURES = {
     "knn_index_search_filter_batch_dev": (ctypes.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp]),
     "knn_index_search_finish_batch_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "knn_index_search_end_dev": (ctypes.c_int, [c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "knn_index_add_typed": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int]),
+    "knn_index_add_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_vp]),
+    "knn_index_search_typed": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp]),
+    "knn_index_search_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp, c_i64, c_vp]),
+    "knn_index_search_begin_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, ctypes.POINTER(c_i64),
+                                                        ctypes.POINTER(c_i64), c_vp]),
+    "knn_index_search_filter_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_i64, c_vp, c_vp]),
+    "knn_index_search_finish_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp, c_vp, c_i64,
+                                                         c_vp]),
     "knn_index_reconstruct": (ctypes.c_int, [c_vp, c_i64, c_i64, c_vp]),
     "knn_merge_topk_dev": (ctypes.c_int, [ctypes.c_int, c_i64, c_i64, ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "knn_peer_buffer_alloc": (ctypes.c_int, [ctypes.POINTER(c_vp), c_i64, ctypes.c_int]),

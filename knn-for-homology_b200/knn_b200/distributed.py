@@ -407,18 +407,23 @@ class ShardedIndexFlat:
         (n, d) float32 matrix on this rank's device, crossing PCIe once in total instead of once per rank: rank r
         uploads rows [r n/G, (r+1) n/G) and one all-gather over NVLink hands every rank the rest (C4 on 8 GPUs: 51 MB
         instead of 410 MB over each rank's PCIe link).  x_host: CPU torch tensor (pinned for an asynchronous copy) or
-        numpy array, float32, C-contiguous.  Collective."""
+        numpy array.  float16 / bfloat16 rows keep their dtype (half the PCIe and NVLink bytes; the index reads them as
+        they are), anything else becomes float32.  Collective."""
         import torch
 
+        from .index import _h16_code
+
         if isinstance(x_host, np.ndarray):
-            x_host = torch.from_numpy(np.ascontiguousarray(x_host, dtype=np.float32))
+            x_host = torch.from_numpy(np.ascontiguousarray(x_host, dtype=None if x_host.dtype == np.float16 else np.float32))
+        elif _h16_code(x_host.dtype) is None:
+            x_host = x_host.to(torch.float32)
         n, d = x_host.shape
         dev = torch.device("cuda", self.local.device) if self._dist.is_initialized() and self._dist.get_backend(self.group) == "nccl" \
             else x_host.device
         if self.world == 1:
             return x_host.to(dev, non_blocking=True).contiguous()
         chunk = -(-n // self.world)  # equal chunks (all_gather_into_tensor); the tail of the last one is padding
-        buf = torch.empty((self.world * chunk, d), dtype=torch.float32, device=dev)
+        buf = torch.empty((self.world * chunk, d), dtype=x_host.dtype, device=dev)
         lo, hi = min(n, self.rank * chunk), min(n, (self.rank + 1) * chunk)
         mine = buf[self.rank * chunk:(self.rank + 1) * chunk]
         if hi > lo:

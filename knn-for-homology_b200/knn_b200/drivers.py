@@ -46,16 +46,19 @@ def _pinned_pair(device: int):
 
 
 def _upload(x: np.ndarray, device: int):
+    """Host matrix -> a device tensor of the same values: float16 stays float16 (half the PCIe bytes; the device
+    up-converts, exactly, where the caller needs float32), any other dtype becomes float32."""
     import torch
 
-    x = np.ascontiguousarray(x, dtype=np.float32)
+    x = np.ascontiguousarray(x, dtype=None if x.dtype == np.float16 else np.float32)
     dev = torch.device("cuda", device)
     if x.nbytes < 2 * _CHUNK_BYTES:
         return torch.from_numpy(x).to(dev)
-    out = torch.empty(x.shape, dtype=torch.float32, device=dev)
-    src, dst = torch.from_numpy(x).view(-1), out.view(-1)
-    n = _CHUNK_BYTES // 4
-    bufs = [b.view(torch.float32) for b in _pinned_pair(device)]
+    src = torch.from_numpy(x)
+    out = torch.empty(x.shape, dtype=src.dtype, device=dev)
+    src, dst = src.view(-1), out.view(-1)
+    n = _CHUNK_BYTES // src.element_size()
+    bufs = [b.view(src.dtype) for b in _pinned_pair(device)]
     done = [torch.cuda.Event(), torch.cuda.Event()]
     for c, i in enumerate(range(0, src.numel(), n)):
         w = c & 1
@@ -112,7 +115,9 @@ def search(embeddings: np.ndarray, hits: int = 10, metric: int = METRIC_INNER_PR
     ``index``: an IndexFlat of the same width and metric to reuse (it is reset first): a loop over many matrices
     then pays for the device storage and the ~1 GB of search workspaces once instead of once per matrix."""
     device = _default_device() if device is None else device
-    x = _upload(embeddings, device)
+    # float16 embeddings cross PCIe as they are and are up-converted on the device (exact): normalisation runs in
+    # float32, as the reference's does after its host-side cast (cath/search.py:39-40)
+    x = _upload(embeddings, device).float()
     if metric == METRIC_INNER_PRODUCT:
         normalize_L2(x)
     if index is None:
@@ -136,8 +141,11 @@ def search_and_save(cath_data: Path, device: int | None = None) -> None:
         hits, scores = {}, {}
         indexes = {}  # one index per embedding width, reused across the files (the embedders differ in width)
         for file_path in sorted(cath_data.glob("*.npy")):
-            # fp16 embeddings of the half precision model are cast to the fp32 the index wants (cath/search.py:39-40)
-            embeddings = np.load(file_path).astype(np.float32)
+            # fp16 embeddings of the half precision model stay fp16 on the host: `search` uploads them as they are and
+            # casts to fp32 on the device, with the same values as the reference's host-side cast (cath/search.py:39-40)
+            embeddings = np.load(file_path)
+            if embeddings.dtype != np.float16:
+                embeddings = embeddings.astype(np.float32)
             print(file_path.stem, embeddings.shape)
             start = time.time()
             if embeddings.shape[1] not in indexes:
@@ -161,13 +169,13 @@ def faiss_search(haystack, queries: np.ndarray, hits: int = 13, metric: int = ME
     import torch
 
     device = _default_device() if device is None else device
-    q = _upload(queries, device)
+    q = _upload(queries, device).float()  # float32 on the device, as the in-place normalisation needs
     if metric == METRIC_INNER_PRODUCT:
         normalize_L2(q)
         _write_back(queries, q)
     writer = None
     if isinstance(haystack, np.ndarray):
-        h = _upload(haystack, device)
+        h = _upload(haystack, device).float()
         if metric == METRIC_INNER_PRODUCT:
             normalize_L2(h)
             if haystack.dtype != np.float32 or not haystack.flags.c_contiguous:
@@ -229,10 +237,12 @@ def proteins_search(full_sequences_data: Path, index_mode: str = "flat", k: int 
     device = _default_device() if device is None else device
     full_sequences_data = Path(full_sequences_data)
     npy = full_sequences_data.joinpath("full_sequences.npy")
-    embeddings = np.load(npy).astype(np.float32)
+    embeddings = np.load(npy)
+    if embeddings.dtype != np.float16:  # fp16 is uploaded as it is and cast on the device (same values, half the bytes)
+        embeddings = embeddings.astype(np.float32)
     print("full_sequences", embeddings.shape)
     start = time.time()
-    x = _upload(embeddings, device)
+    x = _upload(embeddings, device).float()
     normalize_L2(x)
     index = IndexFlat(x.shape[1], METRIC_INNER_PRODUCT, device=device)
     index.train(x)
@@ -277,7 +287,7 @@ def create_index(args=None):
     logger.info(f"Loading database from {args.dir.joinpath('train.npy')}")
     embeddings = np.load(str(args.dir.joinpath("train.npy")))
     logger.info(f"Building exact flat index on {embeddings.shape}")
-    x = _upload(embeddings, device)
+    x = _upload(embeddings, device).float()
     normalize_L2(x)
     index = IndexFlat(x.shape[1], METRIC_INNER_PRODUCT, device=device)
     index.train(x)

@@ -8,6 +8,12 @@ seqvec_search/main.py:22-50): ``normalize_L2``, ``IndexFlat(d, metric)``, ``.tra
 Inputs may be numpy arrays (host path: the library copies H2D/D2H itself) or CUDA
 ``torch.Tensor``s on the index's device (device path: results come back as CUDA tensors on
 the current torch stream).
+
+16-bit rows are read as they are: float16 / bfloat16 CUDA tensors, float16 numpy arrays and
+contiguous float16 / bfloat16 CPU torch tensors (numpy has no bfloat16) are handed to the
+library without an fp32 copy, and every call returns exactly what it returns for the same
+rows up-converted to float32.  Other dtypes are converted to float32 first, as faiss's
+wrapper does.
 """
 from __future__ import annotations
 
@@ -35,6 +41,22 @@ def _default_device() -> int:
     except Exception:
         pass
     return 0
+
+
+def _h16_code(dtype):
+    """KNN_DTYPE code of a 16-bit torch / numpy dtype that the library reads as it is, else None."""
+    if dtype == np.float16:
+        return _lib.DTYPE_F16
+    if type(dtype).__module__.startswith("torch"):
+        import torch
+
+        return {torch.float16: _lib.DTYPE_F16, torch.bfloat16: _lib.DTYPE_BF16}.get(dtype)
+    return None
+
+
+def _is_host_h16_tensor(x) -> bool:
+    """A CPU torch tensor of a 16-bit type: searched and added through the host path (numpy has no bfloat16)."""
+    return _is_torch(x) and not x.is_cuda and _h16_code(x.dtype) is not None
 
 
 def _torch_stream(device: int) -> int:
@@ -121,9 +143,23 @@ class IndexFlat:
         if x.ndim != 2:
             raise ValueError("expected a 2-d array")
         assert x.shape[1] == self.d, "dimension mismatch: got %d, index has %d" % (x.shape[1], self.d)
+        if x.dtype == np.float16:
+            return np.ascontiguousarray(x)  # read as it is (exact up-conversion in the kernels)
         return np.ascontiguousarray(x, dtype=np.float32)  # faiss's python wrapper does the same
 
+    def _host_rows(self, x):
+        """Host rows -> (object that owns them, KNN_DTYPE code, address of the first row)."""
+        if _is_host_h16_tensor(x):
+            if x.dim() != 2:
+                raise ValueError("expected a 2-d tensor")
+            assert x.shape[1] == self.d, "dimension mismatch: got %d, index has %d" % (x.shape[1], self.d)
+            x = x.contiguous()
+            return x, _h16_code(x.dtype), x.data_ptr()
+        x = self._host_matrix(x)
+        return x, _h16_code(x.dtype) or _lib.DTYPE_F32, x.ctypes.data
+
     def _dev_matrix(self, x):
+        """CUDA tensor -> (contiguous tensor, KNN_DTYPE code): float16 / bfloat16 as they are, anything else float32."""
         import torch
 
         if x.dim() != 2:
@@ -131,29 +167,34 @@ class IndexFlat:
         assert x.shape[1] == self.d, "dimension mismatch: got %d, index has %d" % (x.shape[1], self.d)
         if not x.is_cuda or x.device.index != self.device:
             raise ValueError("tensor must live on cuda:%d" % self.device)
-        return x.to(torch.float32).contiguous()
+        code = _h16_code(x.dtype)
+        if code is not None:
+            return x.contiguous(), code
+        return x.to(torch.float32).contiguous(), _lib.DTYPE_F32
 
     # -- faiss methods --------------------------------------------------------------------
     def train(self, x) -> None:
         """No-op for a flat index (pfam/proteins_search.py:35, seqvec_search/main.py:37)."""
         if not _is_torch(x):
             self._host_matrix(x)
+        elif _is_host_h16_tensor(x):
+            self._host_rows(x)
 
     def reserve(self, n: int) -> None:
         _lib.check(self._lib.knn_index_reserve(self._h, int(n)))
 
     def add(self, x) -> None:
         """Append rows; ids are the row numbers (cath/search.py:22)."""
-        if _is_torch(x):
-            x = self._dev_matrix(x)
-            _lib.check(self._lib.knn_index_add_dev(self._h, x.shape[0], x.data_ptr(), _torch_stream(self.device)))
+        if _is_torch(x) and not _is_host_h16_tensor(x):
+            x, code = self._dev_matrix(x)
+            _lib.check(self._lib.knn_index_add_typed_dev(self._h, x.shape[0], x.data_ptr(), code, _torch_stream(self.device)))
             # the ingest kernel reads x asynchronously on the current stream; keep it alive until then
             import torch
 
             x.record_stream(torch.cuda.current_stream(self.device))
             return
-        x = self._host_matrix(x)
-        _lib.check(self._lib.knn_index_add(self._h, x.shape[0], x.ctypes.data))
+        x, code, ptr = self._host_rows(x)
+        _lib.check(self._lib.knn_index_add_typed(self._h, x.shape[0], ptr, code))
 
     def reset(self) -> None:
         _lib.check(self._lib.knn_index_reset(self._h))
@@ -163,18 +204,18 @@ class IndexFlat:
         k = int(k)
         if k <= 0:
             raise ValueError("k must be positive")
-        if _is_torch(x):
+        if _is_torch(x) and not _is_host_h16_tensor(x):
             import torch
 
-            x = self._dev_matrix(x)
+            x, code = self._dev_matrix(x)
             D = torch.empty((x.shape[0], k), dtype=torch.float32, device=x.device)
             I = torch.empty((x.shape[0], k), dtype=torch.int64, device=x.device)
-            _lib.check(self._lib.knn_index_search_dev(self._h, x.shape[0], x.data_ptr(), k, D.data_ptr(), I.data_ptr(),
-                                                      int(id_base), _torch_stream(self.device)))
+            _lib.check(self._lib.knn_index_search_typed_dev(self._h, x.shape[0], x.data_ptr(), code, k, D.data_ptr(),
+                                                            I.data_ptr(), int(id_base), _torch_stream(self.device)))
             return D, I
-        x = self._host_matrix(x)
+        x, code, ptr = self._host_rows(x)
         D, I = _result_arrays(x.shape[0], k)
-        _lib.check(self._lib.knn_index_search(self._h, x.shape[0], x.ctypes.data, k, D.ctypes.data, I.ctypes.data))
+        _lib.check(self._lib.knn_index_search_typed(self._h, x.shape[0], ptr, code, k, D.ctypes.data, I.ctypes.data))
         if id_base:
             I[I >= 0] += int(id_base)
         return D, I
@@ -187,35 +228,37 @@ class IndexFlat:
         element-wise MIN: every shard holds j rows at or above it)."""
         import torch
 
-        x = self._dev_matrix(x)
+        x, code = self._dev_matrix(x)
         lower = torch.empty((x.shape[0],), dtype=torch.float32, device=x.device)
         lower_j = torch.empty_like(lower) if j is not None else None
-        _lib.check(self._lib.knn_index_search_filter_dev(self._h, x.shape[0], x.data_ptr(), int(k), lower.data_ptr(),
-                                                         int(j or 0), lower_j.data_ptr() if j is not None else None,
-                                                         _torch_stream(self.device)))
-        self._pending_x = x  # phase 2 needs the same queries (kept alive here)
+        _lib.check(self._lib.knn_index_search_filter_typed_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
+                                                               lower.data_ptr(), int(j or 0),
+                                                               lower_j.data_ptr() if j is not None else None,
+                                                               _torch_stream(self.device)))
+        self._pending_x = (x, code)  # phase 2 needs the same queries (kept alive here)
         return lower if j is None else (lower, lower_j)
 
     def search_finish(self, lower, k: int, id_base: int = 0):
         """Phase 2: exact rescoring of the candidates that survive the combined bound -> this shard's (D, I)."""
         import torch
 
-        x = self._pending_x
+        x, code = self._pending_x
         self._pending_x = None
         D = torch.empty((x.shape[0], int(k)), dtype=torch.float32, device=x.device)
         I = torch.empty((x.shape[0], int(k)), dtype=torch.int64, device=x.device)
         lower = lower.contiguous()
-        _lib.check(self._lib.knn_index_search_finish_dev(self._h, x.shape[0], x.data_ptr(), int(k), lower.data_ptr(),
-                                                         D.data_ptr(), I.data_ptr(), int(id_base), _torch_stream(self.device)))
+        _lib.check(self._lib.knn_index_search_finish_typed_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
+                                                               lower.data_ptr(), D.data_ptr(), I.data_ptr(), int(id_base),
+                                                               _torch_stream(self.device)))
         return D, I
 
     # -- the same, batch by batch (the caller overlaps exchange + finish of batch b with the filter of batch b + 1) --
     def search_begin(self, x, k: int):
         """Returns (nbatches, batch_rows); x is kept alive until search_end."""
-        x = self._dev_matrix(x)
+        x, code = self._dev_matrix(x)
         nb, rows = ctypes.c_int64(), ctypes.c_int64()
-        _lib.check(self._lib.knn_index_search_begin_dev(self._h, x.shape[0], x.data_ptr(), int(k), ctypes.byref(nb),
-                                                        ctypes.byref(rows), _torch_stream(self.device)))
+        _lib.check(self._lib.knn_index_search_begin_typed_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
+                                                              ctypes.byref(nb), ctypes.byref(rows), _torch_stream(self.device)))
         self._pending_x = x
         return nb.value, rows.value
 
@@ -231,9 +274,9 @@ class IndexFlat:
         _lib.check(self._lib.knn_index_search_end_dev(self._h, D.data_ptr(), I.data_ptr(), int(id_base), _torch_stream(self.device)))
         self._pending_x = None
 
-    def search_into(self, xq_ptr: int, nq: int, k: int, D_ptr: int, I_ptr: int) -> None:
-        """Host-pointer search into caller-owned (e.g. pinned) buffers: the raw C-ABI call."""
-        _lib.check(self._lib.knn_index_search(self._h, int(nq), int(xq_ptr), int(k), int(D_ptr), int(I_ptr)))
+    def search_into(self, xq_ptr: int, nq: int, k: int, D_ptr: int, I_ptr: int, dtype: int = _lib.DTYPE_F32) -> None:
+        """Host-pointer search into caller-owned (e.g. pinned) buffers: the raw C-ABI call (dtype: a KNN_DTYPE code)."""
+        _lib.check(self._lib.knn_index_search_typed(self._h, int(nq), int(xq_ptr), int(dtype), int(k), int(D_ptr), int(I_ptr)))
 
     def reconstruct_n(self, i0: int = 0, n: int | None = None) -> np.ndarray:
         n = self.ntotal - i0 if n is None else n
