@@ -156,6 +156,39 @@ int knn_index_search_finish_batch_dev(knn_index* idx, int64_t b, const float* bo
                                       int64_t id_base, void* stream);
 int knn_index_search_end_dev(knn_index* idx, float* D_dev, int64_t* I_dev, int64_t id_base, void* stream);
 
+/* Filtered search (faiss SearchParameters / IDSelector on IndexFlat): restrict a search to selected rows and exclude one
+ * row per query, inside the kernels.
+ * Contract: a filtered search returns exactly what the unfiltered search returns on an index that holds only the
+ * eligible rows, with ids mapped back to the original row numbers - the same D and I bits (the exact rescoring of a
+ * (query, row) pair does not depend on the other rows, and the mapping preserves the lower-id-first tie rule).
+ *   Row selector (shared by every query of the call): row r is eligible iff allow_bit0 + r < allow_nbits and bit
+ *     allow_bit0 + r of allow_bits is set.  allow_bits is an array of 32-bit words, least significant bit first: its
+ *     byte layout is faiss's IDSelectorBitmap (bit i & 7 of byte i >> 3).  Bits past allow_nbits select nothing;
+ *     allow_bit0 lets one global bitmap serve every shard of a row-sharded database.  NULL: every row is eligible.
+ *   Per-query exclusion: exclude_ids[q] is one id in the space the call returns (row + id_base); that row is never
+ *     returned for query q.  -1, or an id outside the index, excludes nothing.  NULL: no exclusions.
+ * When fewer than k rows remain for a query the tail is padded as for k > ntotal (id -1, -FLT_MAX / +FLT_MAX).  The
+ * statistics keep their meaning.  p == NULL is the unfiltered call.  Negative allow_bit0, allow_nbits or id_base, and
+ * filter arrays in the wrong memory space (device calls: device memory of the index's device; host calls: not device
+ * memory), return KNN_ERR_INVALID.  The host form copies the bitmap words that cover the index and the nq ids to the
+ * device; the device forms read the caller's arrays, which must stay valid until the search is done (for
+ * begin_params: until search_end). */
+typedef struct knn_search_params {
+    const uint32_t* allow_bits; int64_t allow_bit0; int64_t allow_nbits; /* NULL: every row */
+    const int64_t* exclude_ids;                                          /* NULL: none; nq ids, -1 = none */
+} knn_search_params;
+/* index.search(xq, k, params=SearchParameters(sel=...)) on host arrays (ids are row numbers). */
+int knn_index_search_params(knn_index* idx, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I,
+                            const knn_search_params* p);
+int knn_index_search_params_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k, float* D_dev,
+                                int64_t* I_dev, int64_t id_base, const knn_search_params* p, void* stream);
+/* knn_index_search_begin_typed_dev with a filter; the filter_batch, finish_batch and end calls that follow apply it, and
+ * finish_batch and end must be given this id_base (otherwise KNN_ERR_INVALID).  The one-shot search_filter_dev /
+ * search_finish_dev pair has no filtered form. */
+int knn_index_search_begin_params_dev(knn_index* idx, int64_t nq, const void* xq_dev, int dtype, int64_t k, int64_t id_base,
+                                      const knn_search_params* p, int64_t* nbatches_out, int64_t* batch_rows_out,
+                                      void* stream);
+
 /* Copy rows [i0, i0+n) back to the host as float32 (faiss Index::reconstruct_n); feeds
  * write_index (pfam/proteins_search.py:39-40). */
 int knn_index_reconstruct(knn_index* idx, int64_t i0, int64_t n, float* out);

@@ -114,6 +114,50 @@ __host__ __device__ inline float key_score(uint64_t key, int largest) {
 }
 __host__ __device__ inline uint32_t key_id(uint64_t key) { return ~uint32_t(key); }
 
+// ---- filtered search (knn_search_params) --------------------------------------------------
+// Which rows a query may return, in device memory.  Row r is eligible for query q iff
+//   (allow_bits == null || (allow_bit0 + r < allow_nbits && bit allow_bit0 + r of allow_bits is set)) &&
+//   (exclude == null || exclude[q] != r + id_base).
+// The kernels apply it where a candidate is created (GEMM epilogues, the exact path's segment select), never later:
+// every threshold and bound of the tensor path is built from candidates, so an ineligible candidate would move them.
+struct RowFilter {
+    const uint32_t* allow_bits = nullptr;  // LSB first; faiss IDSelectorBitmap byte order
+    int64_t allow_bit0 = 0, allow_nbits = 0;
+    const int64_t* exclude = nullptr;      // one id per query of the launch (-1 or out of range: none)
+    int64_t id_base = 0;                   // the id of row r is r + id_base
+    bool active() const { return allow_bits != nullptr || exclude != nullptr; }
+    RowFilter queries_from(int64_t q0) const {  // the same filter for the queries [q0, ...) of this one
+        RowFilter f = *this;
+        if (f.exclude) f.exclude += q0;
+        return f;
+    }
+};
+// Eligibility bits of rows r0 .. r0 + 31 under the selector (bit i: row r0 + i); the same for every lane of a warp.
+__device__ __forceinline__ uint32_t allow_word(const RowFilter& f, int64_t r0) {
+    if (!f.allow_bits) return ~0u;
+    const int64_t b0 = f.allow_bit0 + r0;
+    const int64_t left = f.allow_nbits - b0;
+    if (left <= 0) return 0u;
+    const int64_t w = b0 >> 5;
+    const int sh = int(b0 & 31);
+    const uint32_t lo = __ldg(f.allow_bits + w);
+    const uint32_t hi = (sh && (w + 1) * 32 < f.allow_nbits) ? __ldg(f.allow_bits + w + 1) : 0u;
+    uint32_t m = __funnelshift_r(lo, hi, sh);
+    if (left < 32) m &= (1u << int(left)) - 1u;
+    return m;
+}
+__device__ __forceinline__ bool row_allowed(const RowFilter& f, int64_t r) {
+    if (!f.allow_bits) return true;
+    const int64_t b = f.allow_bit0 + r;
+    return b < f.allow_nbits && ((__ldg(f.allow_bits + (b >> 5)) >> (b & 31)) & 1u);
+}
+// Row that query q (of the launch) excludes, -1 for none.
+__device__ __forceinline__ int64_t excluded_row(const RowFilter& f, int64_t q) {
+    if (!f.exclude) return -1;
+    const int64_t id = __ldg(f.exclude + q);
+    return id < 0 || id - f.id_base < 0 ? -1 : id - f.id_base;
+}
+
 // ---- kernel launchers (one translation unit each) ---------------------------------------
 struct DbStats {          // device-resident, updated by the ingest kernel with atomicMax on
     unsigned max_norm2;   // float bits (values are >= 0, so the uint order is the float order)
@@ -160,10 +204,11 @@ int launch_rerank(const float* xq_f32, const float* xnorm2, int64_t nq, int dp, 
                   cudaStream_t s);
 
 // select.cu
-// Level 1: dense rows -> per (query, segment) best-k appended to lists[q][seg*k + r].
+// Level 1: dense rows -> per (query, segment) best-k appended to lists[q][seg*k + r].  Column c is row id_base + c;
+// rows that `filt` makes ineligible never enter a list (filt.exclude: one id per query of this launch).
 int launch_select_dense(const float* scores, int64_t ld, int64_t ncols, int64_t nq, int seg_len,
                         uint32_t id_base, int k, int largest, float* list_scores, uint32_t* list_ids,
-                        int64_t list_ld, int64_t list_off, cudaStream_t s);
+                        int64_t list_ld, int64_t list_off, const RowFilter& filt, cudaStream_t s);
 // Final: lists[q][0..len) (len = counts ? min(counts[q], list_ld) : fixed_len) -> sorted D/I rows.
 int launch_select_final(const float* list_scores, const uint32_t* list_ids, const int* counts,
                         int64_t list_ld, int64_t fixed_len, int64_t nq, int k, int largest, float* D,
@@ -196,9 +241,11 @@ int gemm_plan_query_rows_multiple(const GemmPlan* p);     // nq_pad granularity 
 // Scores queries (16-bit, format fmt_q, [nq_pad x dp]) against database rows [j0, j1) (16-bit, format fmt_db,
 // [ntotal x dp]) on the tensor cores and appends every (score, id) with score >= thr[q] to the candidate lists.
 // dense_first: rows are stored at slot (j - j0) without atomics (first panel, thr = -inf).
+// filt (optional): rows it makes ineligible never become candidates (dense panel: NaN score, id kInvalidId, which the
+// tighten and rerank kernels drop); filt.exclude holds one id per query of this launch.
 int gemm_filter_launch(GemmPlan* p, const h16_t* xq_h16, int fmt_q, int64_t nq, int64_t nq_pad, int dp,
                        const h16_t* xb_h16, int fmt_db, int64_t ntotal, const float* ynorm2, int64_t j0,
-                       int64_t j1, int metric, bool dense_first, FilterState st, cudaStream_t s);
+                       int64_t j1, int metric, bool dense_first, FilterState st, const RowFilter& filt, cudaStream_t s);
 // After a panel: thr[q] <- (k-th best approx score so far) - 2*eps[q]; drops candidates below the
 // new threshold; raises *overflow when a list ran past its capacity.
 int launch_tighten(FilterState st, const float* eps, int64_t nq, int k, int compact, float* tau_out,
@@ -216,6 +263,8 @@ int launch_fill_f32(float* p, int64_t n, float v, cudaStream_t s);
 // Overflow repair: out[i] = float(xq[idx[i]]) (rows of d elements of xq_dtype, written as fp32);
 // D[idx[i]] = Dt[i], I[idx[i]] = It[i] (rows of k).
 int launch_gather_rows(const void* xq, int xq_dtype, int d, const int* idx, int64_t n, float* out, cudaStream_t s);
+// out[i] = ids[idx[i]] (the exclusion ids of the queries an overflow repair gathers)
+int launch_gather_ids(const int64_t* ids, const int* idx, int64_t n, int64_t* out, cudaStream_t s);
 int launch_scatter_results(const float* Dt, const int64_t* It, const int* idx, int64_t n, int k, float* D, int64_t* I,
                            cudaStream_t s);
 

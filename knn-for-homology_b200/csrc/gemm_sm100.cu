@@ -20,6 +20,8 @@
 // query tile fastest so that co-resident CTAs share database tiles in L2.
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace knn {
@@ -252,6 +254,20 @@ struct GemmArgs {
     uint32_t idesc;            // tcgen05 instruction descriptor (operand formats of this launch)
     int debug_skip_epilogue;   // experiments only: accumulators are not read (results are then meaningless)
 };
+// Arguments of the filtered instantiations: the unfiltered ones keep GemmArgs (and their code) as it is.
+struct GemmArgsFilt : GemmArgs {
+    RowFilter filt;            // rows that may not become candidates (exclude: one id per query of the launch)
+};
+template <bool FILT> using GemmArgsT = typename std::conditional<FILT, GemmArgsFilt, GemmArgs>::type;
+
+// Eligibility bits of the 32 columns j_first .. j_first + 31 for a query that excludes row ex_row (-1: none).
+__device__ __forceinline__ uint32_t eligible_cols(const RowFilter& f, int64_t j_first, int64_t ex_row) {
+    uint32_t m = allow_word(f, j_first);
+    const int64_t e = ex_row - j_first;
+    if (e >= 0 && e < 32) m &= ~(1u << int(e));
+    return m;
+}
+__device__ __forceinline__ float nan_score() { return __uint_as_float(0x7FC00000u); }
 
 constexpr int kStashEntries = 512;  // per epilogue warp: (score bits, lane << 8 | column in tile)
 
@@ -312,9 +328,9 @@ __device__ __forceinline__ void load_scores(uint32_t taddr, int64_t j_first, con
     }
 }
 
-template <int CG, bool L2, bool DENSE>
+template <int CG, bool L2, bool DENSE, bool FILT>
 __global__ void __launch_bounds__(kThreads, 1)
-gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_db, const GemmArgs args) {
+gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_db, const GemmArgsT<FILT> args) {
     using C = Cfg<CG>;
     const int nstages = args.stages;  // depth of the TMA -> MMA shared-memory ring (<= kMaxStages)
     extern __shared__ uint8_t smem_raw[];
@@ -423,6 +439,8 @@ gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
             const int64_t jbase = args.j0 + int64_t(nt) * BN;
             const bool q_ok = q < args.nq;
             const float thr = q_ok ? args.thr[q] : FLT_MAX;
+            int64_t ex_row = -1;  // lane-local
+            if constexpr (FILT) ex_row = q_ok ? excluded_row(args.filt, q) : -1;
             mbar_wait(&bars->acc_full[acc], acc_phase);
             tc_fence_after();
             const uint32_t taddr = tmem_base + uint32_t(acc * BN) + (uint32_t(quarter * 32) << 16);
@@ -461,6 +479,14 @@ gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                     float v[32];
                     load_scores<L2>(taddr + uint32_t(cg * 32), jbase + cg * 32, args, v);
                     const int64_t j_first = jbase + cg * 32;
+                    // ineligible columns: a NaN score and an invalid id, which tighten and rerank skip and never count
+                    uint32_t ok = ~0u;
+                    if constexpr (FILT) {
+                        ok = eligible_cols(args.filt, j_first, ex_row);
+#pragma unroll
+                        for (int i = 0; i < 32; ++i) v[i] = ((ok >> i) & 1u) ? v[i] : nan_score();
+                    }
+                    auto col_id = [&](int i) { return FILT && !((ok >> i) & 1u) ? kInvalidId : uint32_t(j_first + i); };
                     if (q_ok) {
                         float* cs = args.cand_scores + q * int64_t(args.cap) + (j_first - args.j0);
                         uint32_t* ci = args.cand_ids + q * int64_t(args.cap) + (j_first - args.j0);
@@ -468,15 +494,14 @@ gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
 #pragma unroll
                             for (int i = 0; i < 32; i += 4) {
                                 *reinterpret_cast<float4*>(cs + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-                                *reinterpret_cast<uint4*>(ci + i) = make_uint4(uint32_t(j_first + i), uint32_t(j_first + i + 1),
-                                                                               uint32_t(j_first + i + 2), uint32_t(j_first + i + 3));
+                                *reinterpret_cast<uint4*>(ci + i) = make_uint4(col_id(i), col_id(i + 1), col_id(i + 2), col_id(i + 3));
                             }
                         } else {
 #pragma unroll
                             for (int i = 0; i < 32; ++i) {
                                 if (j_first + i < args.j1) {
                                     cs[i] = v[i];
-                                    ci[i] = uint32_t(j_first + i);
+                                    ci[i] = col_id(i);
                                 }
                             }
                         }
@@ -507,6 +532,8 @@ gemm_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                             for (int i = 0; i < 32; ++i) mask |= (v[i] >= thr) ? (1u << i) : 0u;
                             const int64_t left = args.j1 - (jbase + cg * 32);  // columns of this group inside the panel
                             if (left < 32) mask &= left <= 0 ? 0u : ((1u << int(left)) - 1u);
+                            // the group's bitmap word is the same for the whole warp; the exclusion is this lane's
+                            if constexpr (FILT) mask &= eligible_cols(args.filt, jbase + cg * 32, ex_row);
                         }
                         while (mask) {  // a lane reads back only what it dumped itself
                             const int i = __ffs(int(mask)) - 1;
@@ -575,8 +602,10 @@ struct StreamBarriers {
 };
 
 // nq_cta: query rows resident per CTA (NQT for one CTA, NQT / 2 for a CTA pair)
-static size_t stream_smem_bytes(int nq_cta, int num_kb, int stages) {
-    return 1024 /*align slack*/ + size_t(num_kb) * nq_cta * BK * 2 + size_t(stages) * kStreamBytesA + sizeof(StreamBarriers) + 128 * sizeof(float) + 64;
+// (filt: plus the excluded row of each of the up to 128 queries)
+static size_t stream_smem_bytes(int nq_cta, int num_kb, int stages, bool filt) {
+    return 1024 /*align slack*/ + size_t(num_kb) * nq_cta * BK * 2 + size_t(stages) * kStreamBytesA + sizeof(StreamBarriers) + 128 * sizeof(float) + 64 +
+           (filt ? 128 * sizeof(int64_t) : 0);
 }
 
 // CG = 2 (NQT = 128): a CTA pair works on 256 database rows with tcgen05.mma.cta_group::2 (M = 256, N = 128).  Each
@@ -600,9 +629,9 @@ static size_t stream_smem_bytes(int nq_cta, int num_kb, int stages) {
 // balance; under the power cap (1.3-1.4 GHz) the tensor pipe sets the pace, and the multicast loads' longer latency on a
 // 6-stage ring costs the rest.  Off by default ("stream_quad"); kept because it is the measured answer to "would
 // multicast help".
-template <int NQT, bool L2, bool DENSE, int CG, int NP>
+template <int NQT, bool L2, bool DENSE, int CG, int NP, bool FILT>
 __global__ void __launch_bounds__(kThreads, 1)
-gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_db, const GemmArgs args) {
+gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_db, const GemmArgsT<FILT> args) {
     static_assert(NP == 1 || CG == 2, "two pairs need CTA pairs");
     constexpr int NQ_CTA = NQT / CG;                 // query rows staged by one CTA
     constexpr uint32_t kTmemColsS = NQT * kStreamAcc < 32 ? 32 : NQT * kStreamAcc;
@@ -614,6 +643,7 @@ gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     uint8_t* smem_a = smem + size_t(args.num_kb) * bytes_q_kb;      // [nstages][128 x 64]
     StreamBarriers* bars = reinterpret_cast<StreamBarriers*>(smem_a + size_t(nstages) * kStreamBytesA);
     float* thr_s = reinterpret_cast<float*>(bars + 1);
+    int64_t* ex_s = reinterpret_cast<int64_t*>(thr_s + 128);  // FILT: row each query excludes (-1: none)
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
     const int num_tiles = args.n_tiles;  // tiles of 128 * CG database rows
@@ -646,6 +676,10 @@ gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
     if (warp == kMmaWarp) tmem_alloc<CG>(&bars->tmem_base, kTmemColsS);
     if (threadIdx.x < 128)
         thr_s[threadIdx.x] = (threadIdx.x < NQT && q_base + int(threadIdx.x) < args.nq) ? args.thr[q_base + threadIdx.x] : FLT_MAX;
+    if constexpr (FILT) {
+        if (threadIdx.x < 128)
+            ex_s[threadIdx.x] = (threadIdx.x < NQT && q_base + int(threadIdx.x) < args.nq) ? excluded_row(args.filt, q_base + threadIdx.x) : -1;
+    }
     tc_fence_before();
     if constexpr (CG == 1) __syncthreads(); else cluster_sync_all();
     tc_fence_after();
@@ -723,6 +757,8 @@ gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
         for (int tile = unit; tile < num_tiles; tile += num_units) {
             const int64_t j = args.j0 + int64_t(tile) * (SBM * CG) + int64_t(cta_rank) * SBM + warp * 32 + lane;  // this thread's database row
             const bool row_ok = j < args.j1;
+            bool row_in = true;  // the selector's bit of this lane's row
+            if constexpr (FILT) row_in = row_ok && row_allowed(args.filt, j);
             float yn = 0.f;
             if (L2 && row_ok) yn = __ldg(args.ynorm2 + j);
             mbar_wait(&bars->acc_full[acc], acc_phase);
@@ -740,8 +776,13 @@ gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                             if (c0 + i < nq) {  // lanes of a warp hold consecutive rows: coalesced per query
                                 float v = __uint_as_float(r[i]);
                                 if (L2) v = 2.0f * v - yn;
+                                uint32_t id = uint32_t(j);
+                                if (FILT && !(row_in && ex_s[c0 + i] != j)) {  // ineligible: skipped by tighten and rerank
+                                    v = nan_score();
+                                    id = kInvalidId;
+                                }
                                 args.cand_scores[int64_t(q_base + c0 + i) * args.cap + (j - args.j0)] = v;
-                                args.cand_ids[int64_t(q_base + c0 + i) * args.cap + (j - args.j0)] = uint32_t(j);
+                                args.cand_ids[int64_t(q_base + c0 + i) * args.cap + (j - args.j0)] = id;
                             }
                         }
                     } else {
@@ -751,8 +792,9 @@ gemm_stream_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_const
                             float v = __uint_as_float(r[i]);
                             if (L2) v = 2.0f * v - yn;
                             r[i] = __float_as_uint(v);
-                            mask |= (v >= thr_s[c0 + i]) ? (1u << i) : 0u;  // padding queries carry +FLT_MAX
+                            mask |= (v >= thr_s[c0 + i] && (!FILT || ex_s[c0 + i] != j)) ? (1u << i) : 0u;  // padding queries carry +FLT_MAX
                         }
+                        if (!row_in) mask = 0u;
                         while (mask) {  // rare once the thresholds have tightened
                             const int i = __ffs(int(mask)) - 1;
                             mask &= mask - 1;
@@ -859,9 +901,10 @@ static int make_map(GemmPlan* p, CUtensorMap* map, const h16_t* base, int64_t ro
     return KNN_OK;
 }
 
-template <int CG, bool L2, bool DENSE>
-static int launch_variant(GemmPlan* p, const CUtensorMap& map_q, const CUtensorMap& map_db, const GemmArgs& a, cudaStream_t s) {
-    auto kern = gemm_filter_kernel<CG, L2, DENSE>;
+template <int CG, bool L2, bool DENSE, bool FILT>
+static int launch_variant(GemmPlan* p, const CUtensorMap& map_q, const CUtensorMap& map_db, const GemmArgsFilt& af, cudaStream_t s) {
+    const GemmArgsT<FILT> a = af;
+    auto kern = gemm_filter_kernel<CG, L2, DENSE, FILT>;
     static bool attr_done[64] = {};  // per instantiation and device (function attributes are per device)
     int dev = 0;
     KNN_CHECK_CUDA(cudaGetDevice(&dev));
@@ -896,10 +939,11 @@ static int launch_variant(GemmPlan* p, const CUtensorMap& map_q, const CUtensorM
     return KNN_OK;
 }
 
-template <int NQT, bool L2, bool DENSE, int CG, int NP = 1>
-static int launch_stream_variant(GemmPlan* p, const CUtensorMap& map_q, const CUtensorMap& map_db, const GemmArgs& a, size_t smem,
+template <int NQT, bool L2, bool DENSE, int CG, int NP, bool FILT>
+static int launch_stream_variant(GemmPlan* p, const CUtensorMap& map_q, const CUtensorMap& map_db, const GemmArgsFilt& af, size_t smem,
                                  cudaStream_t s) {
-    auto kern = gemm_stream_kernel<NQT, L2, DENSE, CG, NP>;
+    const GemmArgsT<FILT> a = af;
+    auto kern = gemm_stream_kernel<NQT, L2, DENSE, CG, NP, FILT>;
     static bool attr_done[64] = {};
     int dev = 0;
     KNN_CHECK_CUDA(cudaGetDevice(&dev));
@@ -939,7 +983,7 @@ static int launch_stream_variant(GemmPlan* p, const CUtensorMap& map_q, const CU
 // Few-queries launch: returns KNN_OK and sets *done when the stream kernel took the launch.
 static int try_stream_launch(GemmPlan* p, const h16_t* xq_h16, int fmt, int64_t nq, int64_t nq_pad, int dp, const h16_t* xb_h16,
                              int64_t ntotal, const float* ynorm2, int64_t j0, int64_t j1, int metric, bool dense_first,
-                             FilterState st, cudaStream_t s, bool* done) {
+                             FilterState st, const RowFilter& filt, cudaStream_t s, bool* done) {
     *done = false;
     if (!p->stream_kernel || nq > 256 || nq_pad < 256 || dp % BK != 0) return KNN_OK;
     if (nq > 64 && !p->stream_pair) return KNN_OK;
@@ -949,13 +993,14 @@ static int try_stream_launch(GemmPlan* p, const h16_t* xq_h16, int fmt, int64_t 
     const int cg = nqt == 128 ? 2 : 1;  // 128 queries: a CTA pair, each CTA keeps 64 of them resident
     const int nq_cta = nqt / cg;
     const int num_kb = dp / BK;
+    const bool filtered = filt.active();
     int stages = kStreamMaxStages;
-    while (stages >= 4 && stream_smem_bytes(nq_cta, num_kb, stages) > size_t(227 * 1024)) --stages;
+    while (stages >= 4 && stream_smem_bytes(nq_cta, num_kb, stages, filtered) > size_t(227 * 1024)) --stages;
     if (stages < 4) return KNN_OK;  // the resident queries leave no room for a ring: the main kernel takes it
     CUtensorMap map_q, map_db;
     KNN_CHECK(make_map(p, &map_q, xq_h16, nq_pad, dp, nq_cta));
     KNN_CHECK(make_map(p, &map_db, xb_h16, ntotal, dp, np == 2 ? SBM / 2 : SBM));  // two pairs: each CTA loads half of its rows
-    GemmArgs a;
+    GemmArgsFilt a;
     a.nq = nq;
     a.m_tiles = 1;
     a.n_tiles = int((j1 - j0 + SBM * cg - 1) / (SBM * cg));
@@ -973,32 +1018,30 @@ static int try_stream_launch(GemmPlan* p, const h16_t* xq_h16, int fmt, int64_t 
     a.stages = stages;
     a.hint_q = kEvictNormal;
     a.hint_db = kEvictNormal;
-    const size_t smem = stream_smem_bytes(nq_cta, num_kb, stages);
+    a.filt = filt;
+    const size_t smem = stream_smem_bytes(nq_cta, num_kb, stages, filtered);
     const bool l2 = metric == KNN_METRIC_L2;
     *done = true;
-#define KNN_STREAM_DISPATCH(NQTV, CGV)                                                                                \
+#define KNN_STREAM_DISPATCH(NQTV, CGV, NPV, F)                                                                         \
     if (l2) {                                                                                                          \
-        return dense_first ? launch_stream_variant<NQTV, true, true, CGV>(p, map_q, map_db, a, smem, s)                \
-                           : launch_stream_variant<NQTV, true, false, CGV>(p, map_q, map_db, a, smem, s);              \
+        return dense_first ? launch_stream_variant<NQTV, true, true, CGV, NPV, F>(p, map_q, map_db, a, smem, s)        \
+                           : launch_stream_variant<NQTV, true, false, CGV, NPV, F>(p, map_q, map_db, a, smem, s);      \
     } else {                                                                                                           \
-        return dense_first ? launch_stream_variant<NQTV, false, true, CGV>(p, map_q, map_db, a, smem, s)               \
-                           : launch_stream_variant<NQTV, false, false, CGV>(p, map_q, map_db, a, smem, s);             \
+        return dense_first ? launch_stream_variant<NQTV, false, true, CGV, NPV, F>(p, map_q, map_db, a, smem, s)       \
+                           : launch_stream_variant<NQTV, false, false, CGV, NPV, F>(p, map_q, map_db, a, smem, s);     \
     }
-    if (np == 2) {
-        if (l2) {
-            return dense_first ? launch_stream_variant<128, true, true, 2, 2>(p, map_q, map_db, a, smem, s)
-                               : launch_stream_variant<128, true, false, 2, 2>(p, map_q, map_db, a, smem, s);
-        }
-        return dense_first ? launch_stream_variant<128, false, true, 2, 2>(p, map_q, map_db, a, smem, s)
-                           : launch_stream_variant<128, false, false, 2, 2>(p, map_q, map_db, a, smem, s);
+    if (filtered) {
+        if (np == 2) { KNN_STREAM_DISPATCH(128, 2, 2, true) }
+        if (nqt == 32) { KNN_STREAM_DISPATCH(32, 1, 1, true) } else if (nqt == 64) { KNN_STREAM_DISPATCH(64, 1, 1, true) } else { KNN_STREAM_DISPATCH(128, 2, 1, true) }
     }
-    if (nqt == 32) { KNN_STREAM_DISPATCH(32, 1) } else if (nqt == 64) { KNN_STREAM_DISPATCH(64, 1) } else { KNN_STREAM_DISPATCH(128, 2) }
+    if (np == 2) { KNN_STREAM_DISPATCH(128, 2, 2, false) }
+    if (nqt == 32) { KNN_STREAM_DISPATCH(32, 1, 1, false) } else if (nqt == 64) { KNN_STREAM_DISPATCH(64, 1, 1, false) } else { KNN_STREAM_DISPATCH(128, 2, 1, false) }
 #undef KNN_STREAM_DISPATCH
 }
 
 int gemm_filter_launch(GemmPlan* p, const h16_t* xq_h16, int fmt_q, int64_t nq, int64_t nq_pad, int dp,
                        const h16_t* xb_h16, int fmt_db, int64_t ntotal, const float* ynorm2, int64_t j0, int64_t j1,
-                       int metric, bool dense_first, FilterState st, cudaStream_t s) {
+                       int metric, bool dense_first, FilterState st, const RowFilter& filt, cudaStream_t s) {
     if (j1 <= j0 || nq <= 0) return KNN_OK;
     // small_m128 (experiments, off): 65..128 queries on single-CTA tiles (M = 128) instead of padding them to a CTA
     // pair's M = 256.  Measured slower (4 stages of 48 KB cover less latency than the pair's 6 x 32 KB).
@@ -1013,13 +1056,13 @@ int gemm_filter_launch(GemmPlan* p, const h16_t* xq_h16, int fmt_q, int64_t nq, 
     }
     if (fmt_q == fmt_db) {
         bool done = false;
-        KNN_CHECK(try_stream_launch(p, xq_h16, fmt_q, nq, nq_pad, dp, xb_h16, ntotal, ynorm2, j0, j1, metric, dense_first, st, s, &done));
+        KNN_CHECK(try_stream_launch(p, xq_h16, fmt_q, nq, nq_pad, dp, xb_h16, ntotal, ynorm2, j0, j1, metric, dense_first, st, filt, s, &done));
         if (done) return KNN_OK;
     }
     CUtensorMap map_q, map_db;
     KNN_CHECK(make_map(p, &map_q, xq_h16, nq_pad, dp, BM));
     KNN_CHECK(make_map(p, &map_db, xb_h16, ntotal, dp, BN / cg));
-    GemmArgs a;
+    GemmArgsFilt a;
     a.nq = nq;
     a.m_tiles = int(nq_pad / (BM * cg));
     a.n_tiles = int((j1 - j0 + BN - 1) / BN);
@@ -1042,16 +1085,20 @@ int gemm_filter_launch(GemmPlan* p, const h16_t* xq_h16, int fmt_q, int64_t nq, 
     if (p->stages >= 2 && p->stages <= (cg == 1 ? 4 : kMaxStages)) a.stages = p->stages;
     a.hint_q = p->l2_hints ? kEvictLast : kEvictNormal;
     a.hint_db = p->l2_hints ? kEvictFirst : kEvictNormal;
+    a.filt = filt;
     const bool l2 = metric == KNN_METRIC_L2;
-#define KNN_GEMM_DISPATCH(CGV)                                                                        \
+#define KNN_GEMM_DISPATCH(CGV, F)                                                                     \
     if (l2) {                                                                                         \
-        return dense_first ? launch_variant<CGV, true, true>(p, map_q, map_db, a, s)                  \
-                           : launch_variant<CGV, true, false>(p, map_q, map_db, a, s);                \
+        return dense_first ? launch_variant<CGV, true, true, F>(p, map_q, map_db, a, s)               \
+                           : launch_variant<CGV, true, false, F>(p, map_q, map_db, a, s);             \
     } else {                                                                                          \
-        return dense_first ? launch_variant<CGV, false, true>(p, map_q, map_db, a, s)                 \
-                           : launch_variant<CGV, false, false>(p, map_q, map_db, a, s);               \
+        return dense_first ? launch_variant<CGV, false, true, F>(p, map_q, map_db, a, s)              \
+                           : launch_variant<CGV, false, false, F>(p, map_q, map_db, a, s);            \
     }
-    if (cg == 1) { KNN_GEMM_DISPATCH(1) } else { KNN_GEMM_DISPATCH(2) }
+    if (filt.active()) {
+        if (cg == 1) { KNN_GEMM_DISPATCH(1, true) } else { KNN_GEMM_DISPATCH(2, true) }
+    }
+    if (cg == 1) { KNN_GEMM_DISPATCH(1, false) } else { KNN_GEMM_DISPATCH(2, false) }
 #undef KNN_GEMM_DISPATCH
 }
 

@@ -217,6 +217,8 @@ struct knn_index {
     // workspaces: exact path / staging
     DevBuf stage, xq_f32, xnorm2, eps, scores, lists_s, lists_i, overflow;
     DevBuf ovf_q, ovf_idx, ovf_x, ovf_D, ovf_I;  // per-query overflow flags of a call and the repair staging
+    DevBuf ovf_ex;                               // exclusion ids of the repaired queries
+    DevBuf f_bits, f_ex;                         // device copies of a host-pointer search's filter (knn_search_params)
     DevBuf h_xq, h_D, h_I;
     // host-pointer search, pipelined per query batch (HostPipe below): two slots of device staging, pinned bounce
     // buffers for pageable caller memory, one copy stream per direction
@@ -247,6 +249,9 @@ struct knn_index {
         const void* xq = nullptr;    // the caller's queries (kept alive by the caller until search_end) ...
         int dtype = KNN_DTYPE_F32;   // ... and their element type
         long long launches0 = 0;
+        bool filtered = false;       // begun by knn_index_search_begin_params_dev with a filter:
+        RowFilter filt;              // its arrays (the caller's, valid until search_end) ...
+        int64_t id_base = 0;         // ... and the id base that finish_batch and end must repeat
     } pend;
     // parameters
     int path_param = 0;
@@ -430,8 +435,9 @@ int prepare_shadow(knn_index* ix, int64_t k, cudaStream_t s) {
 }
 
 // ---- exact path ---------------------------------------------------------------------------
+// filt: which rows each query may return (filt.exclude: one id per query of xq_dev)
 int search_exact(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k, float* D, int64_t* I, int64_t id_base,
-                 cudaStream_t s) {
+                 const RowFilter& filt, cudaStream_t s) {
     const int largest = ix->metric == KNN_METRIC_INNER_PRODUCT;
     const int64_t N = ix->ntotal;
     const int seg_len = 32768;
@@ -459,7 +465,7 @@ int search_exact(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k, 
                                       bf16_rows(ix), ix->ynorm2, j0, j1, ix->metric, ix->scores.as<float>(), chunk, s));
             KNN_CHECK(launch_select_dense(ix->scores.as<float>(), chunk, j1 - j0, nb, seg_len, uint32_t(j0), k, largest,
                                           ix->lists_s.as<float>(), ix->lists_i.as<uint32_t>(), list_ld,
-                                          (j0 / seg_len) * k, s));
+                                          (j0 / seg_len) * k, filt.queries_from(q0), s));
         }
         KNN_CHECK(launch_select_final(ix->lists_s.as<float>(), ix->lists_i.as<uint32_t>(), nullptr, list_ld, list_ld,
                                       nb, k, largest, D + q0 * k, I + q0 * k, id_base, s));
@@ -518,8 +524,9 @@ int tensor_prepare(knn_index* ix) {
 // Filter phase of one query batch (rows [off, off+nb) of W): tensor-core scores over database panels of
 // growing size, survivors appended to the candidate lists, thresholds tightened after every panel.
 // On return thr[q] = (k-th best approximate score) - 2 eps[q].
+// filt: the filter of this batch's queries
 int tensor_filter_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int64_t nb, const void* xq_batch, int qdt, int k,
-                        int cap, int* d_overflow, int* d_ovf_q, cudaStream_t s) {
+                        int cap, int* d_overflow, int* d_ovf_q, const RowFilter& filt, cudaStream_t s) {
     const int64_t N = ix->ntotal;
     const int64_t nb_pad = round_up(nb, 256);
     // first panel: stored densely (every score), sized so that the list it leaves fits the register-resident
@@ -554,7 +561,7 @@ int tensor_filter_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int6
             cudaEventRecord(e0, s);
         }
         KNN_CHECK(gemm_filter_launch(ix->plan, xq_h16, fmt_q, nb, nb_pad, ix->dp, ix->xb_h16, ix->shadow_fmt, N, ix->ynorm2, j0, j1,
-                                     ix->metric, panel == 0, st, s));
+                                     ix->metric, panel == 0, st, filt, s));
         if (ix->profile) cudaEventRecord(e1, s);
         ix->st_gemm_launches++;
         KNN_CHECK(launch_tighten(st, W.eps.as<float>() + off, nb, k, 1, nullptr, d_overflow, s));
@@ -582,8 +589,18 @@ int tensor_finish_batch(knn_index* ix, knn_index::TensorWs& W, int64_t off, int6
     return KNN_OK;
 }
 
+// The exclusion ids of the repaired queries are gathered with them (filt.exclude: one id per query of xq_dev, device).
+int redo_filter(knn_index* ix, const RowFilter& filt, int64_t n, RowFilter* out, cudaStream_t s) {
+    *out = filt;
+    if (!filt.exclude) return KNN_OK;
+    KNN_CHECK(ix->ovf_ex.ensure(sizeof(int64_t) * size_t(n)));
+    KNN_CHECK(launch_gather_ids(filt.exclude, ix->ovf_idx.as<int>(), n, ix->ovf_ex.as<int64_t>(), s));
+    out->exclude = ix->ovf_ex.as<int64_t>();
+    return KNN_OK;
+}
+
 int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const void* xq_dev, int qdt, int k, float* D,
-                    int64_t* I, int64_t id_base, cudaStream_t s) {
+                    int64_t* I, int64_t id_base, const RowFilter& filt, cudaStream_t s) {
     // A candidate list that ran past its capacity (heavily duplicated / clustered scores) is never truncated
     // silently: exactly the queries it happened to are redone with the exact scan and their rows replaced.
     std::vector<int> h_overflow(size_t(nbatches), 0);
@@ -613,7 +630,9 @@ int redo_overflowed(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, con
         KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_idx.p, redo.data() + c0, sizeof(int) * size_t(n), cudaMemcpyHostToDevice, s));
         // the flagged rows are gathered as fp32 (exact for 16-bit queries): the scan sees the values it would have seen
         KNN_CHECK(launch_gather_rows(xq_dev, qdt, ix->d, ix->ovf_idx.as<int>(), n, ix->ovf_x.as<float>(), s));
-        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, KNN_DTYPE_F32, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), id_base, s));
+        RowFilter g;
+        KNN_CHECK(redo_filter(ix, filt, n, &g, s));
+        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, KNN_DTYPE_F32, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), id_base, g, s));
         KNN_CHECK(launch_scatter_results(ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), ix->ovf_idx.as<int>(), n, k, D, I, s));
         KNN_CHECK_CUDA(cudaStreamSynchronize(s));  // `redo` chunk consumed
     }
@@ -710,8 +729,9 @@ struct HostPipe {
 
 // Overflow repair of a host-pointer search: the flagged queries (rare: heavily duplicated rows, out-of-range data) are
 // uploaded again, answered by the exact scan and written into the caller's rows.
+// filt: the call's filter in device memory (ids without an id base)
 int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches, const void* xq, int qdt, int k, float* D,
-                         int64_t* I, cudaStream_t s) {
+                         int64_t* I, const RowFilter& filt, cudaStream_t s) {
     std::vector<int> h_overflow(size_t(nbatches), 0);
     KNN_CHECK_CUDA(cudaMemcpyAsync(h_overflow.data(), ix->overflow.p, sizeof(int) * size_t(nbatches), cudaMemcpyDeviceToHost, s));
     KNN_CHECK_CUDA(cudaStreamSynchronize(s));
@@ -741,7 +761,13 @@ int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches
         hx.resize(size_t(n) * row_bytes);
         for (int64_t i = 0; i < n; ++i) memcpy(hx.data() + i * row_bytes, row_at(xq, redo[c0 + size_t(i)], ix->d, qdt), row_bytes);
         KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_x.p, hx.data(), hx.size(), cudaMemcpyHostToDevice, s));
-        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, qdt, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), 0, s));
+        RowFilter g = filt;
+        if (filt.exclude) {
+            KNN_CHECK(ix->ovf_idx.ensure(sizeof(int) * size_t(chunk)));
+            KNN_CHECK_CUDA(cudaMemcpyAsync(ix->ovf_idx.p, redo.data() + c0, sizeof(int) * size_t(n), cudaMemcpyHostToDevice, s));
+            KNN_CHECK(redo_filter(ix, filt, n, &g, s));
+        }
+        KNN_CHECK(search_exact(ix, n, ix->ovf_x.p, qdt, k, ix->ovf_D.as<float>(), ix->ovf_I.as<int64_t>(), 0, g, s));
         hD.resize(size_t(n) * k);
         hI.resize(size_t(n) * k);
         KNN_CHECK_CUDA(cudaMemcpyAsync(hD.data(), ix->ovf_D.p, sizeof(float) * hD.size(), cudaMemcpyDeviceToHost, s));
@@ -757,7 +783,7 @@ int redo_overflowed_host(knn_index* ix, int64_t nq, int64_t qb, int64_t nbatches
 
 // `hp` (host-pointer search): xq_dev / D / I are then HOST pointers that only the pipe touches.
 int search_tensor(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k, float* D, int64_t* I, int64_t id_base,
-                  cudaStream_t s, HostPipe* hp = nullptr) {
+                  const RowFilter& filt, cudaStream_t s, HostPipe* hp = nullptr) {
     const int cap = candidate_capacity(k, ix->ntotal, ix->dense_small_db != 0);
     int64_t qb = ix->query_batch;
     if (qb > nq) qb = nq;
@@ -803,7 +829,8 @@ int search_tensor(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k,
         int64_t* I_b = hp ? nullptr : I + q0 * k;
         if (hp) KNN_CHECK(hp->acquire(b, q0, nb, s, &xq_b, &D_b, &I_b));
         if (overlap && b >= 2) KNN_CHECK_CUDA(cudaStreamWaitEvent(s, ix->ev_finished[w], 0));  // ws1[w] is free again
-        KNN_CHECK(tensor_filter_batch(ix, ix->ws1[w], 0, nb, xq_b, qdt, k, cap, ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, s));
+        KNN_CHECK(tensor_filter_batch(ix, ix->ws1[w], 0, nb, xq_b, qdt, k, cap, ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0,
+                                      filt.queries_from(q0), s));
         if (hp) {
             KNN_CHECK(hp->filtered(b, s));
             KNN_CHECK(hp->before_finish(b));
@@ -827,9 +854,9 @@ int search_tensor(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int k,
     }
     if (hp) {
         KNN_CHECK(hp->finish());
-        return redo_overflowed_host(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, s);
+        return redo_overflowed_host(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, filt, s);
     }
-    return redo_overflowed(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, id_base, s);
+    return redo_overflowed(ix, nq, qb, nbatches, xq_dev, qdt, k, D, I, id_base, filt, s);
 }
 
 bool use_tensor_path(const knn_index* ix, int64_t nq, int k) {
@@ -839,7 +866,7 @@ bool use_tensor_path(const knn_index* ix, int64_t nq, int k) {
 }
 
 int search_dev_impl(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int64_t k64, float* D, int64_t* I, int64_t id_base,
-                    cudaStream_t s, HostPipe* hp = nullptr) {
+                    cudaStream_t s, HostPipe* hp = nullptr, const RowFilter& filt = RowFilter()) {
     if (nq < 0 || k64 <= 0 || (nq > 0 && (!xq_dev || !D || !I))) {
         set_error("search: invalid arguments (nq=%lld, k=%lld)", (long long)nq, (long long)k64);
         return KNN_ERR_INVALID;
@@ -876,8 +903,8 @@ int search_dev_impl(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int6
             set_error("internal: host pipe on the exact path");
             return KNN_ERR_INVALID;
         }
-        rc = tensor ? search_tensor(ix, nq, xq_dev, qdt, k, D, I, id_base, s, hp)
-                    : search_exact(ix, nq, xq_dev, qdt, k, D, I, id_base, s);
+        rc = tensor ? search_tensor(ix, nq, xq_dev, qdt, k, D, I, id_base, filt, s, hp)
+                    : search_exact(ix, nq, xq_dev, qdt, k, D, I, id_base, filt, s);
     }
     if (rc != KNN_OK) return rc;
     KNN_CHECK_CUDA(cudaEventRecord(ix->search_event, s));
@@ -886,6 +913,64 @@ int search_dev_impl(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int6
         collect_profile(ix);
     }
     ix->st_launches = g_launches.load() - launches0;
+    return KNN_OK;
+}
+
+// ---- filtered search: knn_search_params -> RowFilter --------------------------------------------
+// cudaMemoryTypeUnregistered / Host / Device / Managed of p
+cudaMemoryType memory_type(const void* p) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return cudaMemoryTypeUnregistered;
+    }
+    return a.type;
+}
+
+// Checks the caller's parameters and fills `out`.  Device calls (host = false) take the caller's device arrays as
+// they are: they must be memory of the index's device.  Host calls take host arrays: the words of the bitmap that
+// cover this index's rows and the nq exclusion ids are copied to the device on `s` (the bitmap rebased to them).
+int make_filter(knn_index* ix, const knn_search_params* p, int64_t nq, int64_t id_base, bool host, cudaStream_t s,
+                RowFilter* out, const char* who) {
+    *out = RowFilter();
+    if (!p) return KNN_OK;
+    if (p->allow_bit0 < 0 || p->allow_nbits < 0 || id_base < 0) {
+        set_error("%s: allow_bit0 (%lld), allow_nbits (%lld) and id_base (%lld) must not be negative", who,
+                  (long long)p->allow_bit0, (long long)p->allow_nbits, (long long)id_base);
+        return KNN_ERR_INVALID;
+    }
+    for (const void* a : {static_cast<const void*>(p->allow_bits), static_cast<const void*>(p->exclude_ids)}) {
+        if (!a) continue;
+        const cudaMemoryType t = memory_type(a);
+        const bool dev_mem = t == cudaMemoryTypeDevice || t == cudaMemoryTypeManaged;
+        if (host ? t == cudaMemoryTypeDevice : (!dev_mem || device_of_pointer(a) != ix->device)) {
+            set_error("%s: the filter arrays of a %s call must be %s", who, host ? "host" : "device",
+                      host ? "host memory" : "device memory of the index's device");
+            return KNN_ERR_INVALID;
+        }
+    }
+    out->id_base = id_base;
+    out->allow_bit0 = p->allow_bit0;
+    out->allow_nbits = p->allow_nbits;
+    out->allow_bits = p->allow_bits;
+    out->exclude = p->exclude_ids;
+    if (!host) return KNN_OK;
+    if (p->allow_bits) {
+        // bits [allow_bit0, end) can select a row of this index; a bitmap that covers none of them selects nothing
+        const int64_t end = std::min(p->allow_nbits, p->allow_bit0 + ix->ntotal);
+        const int64_t w0 = p->allow_bit0 >> 5, w1 = end > p->allow_bit0 ? (end + 31) >> 5 : w0;
+        KNN_CHECK(ix->f_bits.ensure(sizeof(uint32_t) * size_t(std::max<int64_t>(1, w1 - w0))));
+        if (w1 > w0)
+            KNN_CHECK_CUDA(cudaMemcpyAsync(ix->f_bits.p, p->allow_bits + w0, sizeof(uint32_t) * size_t(w1 - w0), cudaMemcpyHostToDevice, s));
+        out->allow_bits = ix->f_bits.as<uint32_t>();
+        out->allow_bit0 = p->allow_bit0 - 32 * w0;
+        out->allow_nbits = w1 > w0 ? end - 32 * w0 : 0;
+    }
+    if (p->exclude_ids && nq > 0) {
+        KNN_CHECK(ix->f_ex.ensure(sizeof(int64_t) * size_t(nq)));
+        KNN_CHECK_CUDA(cudaMemcpyAsync(ix->f_ex.p, p->exclude_ids, sizeof(int64_t) * size_t(nq), cudaMemcpyHostToDevice, s));
+        out->exclude = ix->f_ex.as<int64_t>();
+    }
     return KNN_OK;
 }
 
@@ -1010,7 +1095,8 @@ int knn_index_free(knn_index* ix) {
     if (ix->side) cudaStreamSynchronize(ix->side);
     if (ix->hi) cudaStreamSynchronize(ix->hi);
     for (DevBuf* b : {&ix->stage, &ix->xq_f32, &ix->xnorm2, &ix->eps, &ix->scores, &ix->lists_s, &ix->lists_i,
-                      &ix->overflow, &ix->ovf_q, &ix->ovf_idx, &ix->ovf_x, &ix->ovf_D, &ix->ovf_I, &ix->h_xq, &ix->h_D, &ix->h_I})
+                      &ix->overflow, &ix->ovf_q, &ix->ovf_idx, &ix->ovf_x, &ix->ovf_D, &ix->ovf_I, &ix->ovf_ex, &ix->f_bits, &ix->f_ex,
+                      &ix->h_xq, &ix->h_D, &ix->h_I})
         b->release();
     for (int i = 0; i < 2; ++i) {
         ix->hp_xq[i].release(); ix->hp_D[i].release(); ix->hp_I[i].release();
@@ -1159,7 +1245,8 @@ int knn_index_search_dev(knn_index* ix, int64_t nq, const float* xq_dev, int64_t
     return knn_index_search_typed_dev(ix, nq, xq_dev, KNN_DTYPE_F32, k, D_dev, I_dev, id_base, stream);
 }
 
-int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I) {
+static int search_host_impl(knn_index* ix, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I,
+                            const knn_search_params* params) {
     if (!ix || nq < 0 || k <= 0 || (nq > 0 && (!xq || !D || !I))) {
         set_error("search: invalid arguments (nq=%lld, k=%lld)", (long long)nq, (long long)k);
         return KNN_ERR_INVALID;
@@ -1169,12 +1256,15 @@ int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype,
         set_error("search: k=%lld exceeds KNN_MAX_K=%d", (long long)k, KNN_MAX_K);
         return KNN_ERR_LIMIT;
     }
-    if (nq == 0) return KNN_OK;
     DeviceGuard g(ix->device);
+    RowFilter filt;  // ids without an id base: the host forms return row numbers
+    KNN_CHECK(make_filter(ix, params, nq, 0, /*host=*/true, ix->stream, &filt, "search"));
+    if (nq == 0) return KNN_OK;
     if (ix->ntotal > 0 && use_tensor_path(ix, nq, int(k))) {
-        // tensor path: one pipelined pass over the query batches (copies under compute, see HostPipe)
+        // tensor path: one pipelined pass over the query batches (copies under compute, see HostPipe); the filter's
+        // device copy is sliced with the batches
         HostPipe hp{ix, xq, dtype, D, I, int(k), host_pointer_is_pinned(xq), host_pointer_is_pinned(D) && host_pointer_is_pinned(I)};
-        const int rc = search_dev_impl(ix, nq, xq, dtype, k, D, I, 0, ix->stream, &hp);
+        const int rc = search_dev_impl(ix, nq, xq, dtype, k, D, I, 0, ix->stream, &hp, filt);
         if (rc != KNN_OK) {
             // copies into / out of the caller's arrays may still be in flight on the copy streams: nothing may touch
             // the caller's memory once this call has returned, error or not
@@ -1197,7 +1287,8 @@ int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype,
     for (int64_t q0 = 0; q0 < nq; q0 += hb) {
         const int64_t nb = nq - q0 < hb ? nq - q0 : hb;
         KNN_CHECK_CUDA(cudaMemcpyAsync(ix->h_xq.p, row_at(xq, q0, ix->d, dtype), size_t(nb) * row_bytes, cudaMemcpyHostToDevice, ix->stream));
-        KNN_CHECK(search_dev_impl(ix, nb, ix->h_xq.p, dtype, k, ix->h_D.as<float>(), ix->h_I.as<int64_t>(), 0, ix->stream));
+        KNN_CHECK(search_dev_impl(ix, nb, ix->h_xq.p, dtype, k, ix->h_D.as<float>(), ix->h_I.as<int64_t>(), 0, ix->stream, nullptr,
+                                  filt.queries_from(q0)));
         KNN_CHECK_CUDA(cudaMemcpyAsync(D + q0 * k, ix->h_D.p, size_t(nb) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
         KNN_CHECK_CUDA(cudaMemcpyAsync(I + q0 * k, ix->h_I.p, size_t(nb) * k * sizeof(int64_t), cudaMemcpyDeviceToHost, ix->stream));
         KNN_CHECK_CUDA(cudaStreamSynchronize(ix->stream));
@@ -1215,6 +1306,28 @@ int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype,
     return KNN_OK;
 }
 
+int knn_index_search_typed(knn_index* ix, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I) {
+    return search_host_impl(ix, nq, xq, dtype, k, D, I, nullptr);
+}
+
+int knn_index_search_params(knn_index* ix, int64_t nq, const void* xq, int dtype, int64_t k, float* D, int64_t* I,
+                            const knn_search_params* p) {
+    return search_host_impl(ix, nq, xq, dtype, k, D, I, p);
+}
+
+int knn_index_search_params_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k, float* D_dev,
+                                int64_t* I_dev, int64_t id_base, const knn_search_params* p, void* stream) {
+    if (!ix) {
+        set_error("search: null index");
+        return KNN_ERR_INVALID;
+    }
+    DeviceGuard g(ix->device);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    RowFilter filt;
+    KNN_CHECK(make_filter(ix, p, nq, id_base, /*host=*/false, s, &filt, "search"));
+    return search_dev_impl(ix, nq, xq_dev, dtype, k, D_dev, I_dev, id_base, s, nullptr, filt);
+}
+
 int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, float* D, int64_t* I) {
     return knn_index_search_typed(ix, nq, xq, KNN_DTYPE_F32, k, D, I);
 }
@@ -1223,11 +1336,14 @@ int knn_index_search(knn_index* ix, int64_t nq, const float* xq, int64_t k, floa
 // begin -> per batch: filter_batch ... (caller combines the bounds of all shards) ... finish_batch -> end.
 // The batch-wise calls let the caller run exchange + finish of batch b on another stream under the filter of batch
 // b + 1 (knn_b200/distributed.py); knn_index_search_filter_dev / _finish_dev are the all-batches-at-once form.
-static int two_phase_begin(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int64_t k64, cudaStream_t s, const char* who) {
+static int two_phase_begin(knn_index* ix, int64_t nq, const void* xq_dev, int qdt, int64_t k64, cudaStream_t s, const char* who,
+                           const knn_search_params* params = nullptr, int64_t id_base = 0) {
     if (!ix || nq <= 0 || k64 <= 0 || !xq_dev) {
         set_error("%s: invalid arguments", who);
         return KNN_ERR_INVALID;
     }
+    RowFilter filt;
+    KNN_CHECK(make_filter(ix, params, nq, id_base, /*host=*/false, s, &filt, who));
     KNN_CHECK(check_dtype(qdt, who));
     if (k64 > KNN_MAX_K) {
         set_error("%s: k=%lld exceeds KNN_MAX_K=%d", who, (long long)k64, KNN_MAX_K);
@@ -1253,6 +1369,9 @@ static int two_phase_begin(knn_index* ix, int64_t nq, const void* xq_dev, int qd
     P.xq = xq_dev;
     P.dtype = qdt;
     P.launches0 = g_launches.load();
+    P.filtered = params != nullptr;
+    P.filt = filt;
+    P.id_base = id_base;
     P.tensor = ix->ntotal > 0 && use_tensor_path(ix, nq, k);
     ix->last_path = P.tensor ? 2 : 1;
     // The batch geometry depends on nq and query_batch alone, never on the path: the shards of one search lay out
@@ -1294,7 +1413,7 @@ static int two_phase_filter_batch(knn_index* ix, int64_t b, float* lower_b, int6
         return KNN_OK;
     }
     KNN_CHECK(tensor_filter_batch(ix, ix->ws2, q0, nb, row_at(P.xq, q0, ix->d, P.dtype), P.dtype, P.k, P.cap,
-                                  ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, s));
+                                  ix->overflow.as<int>() + b, ix->ovf_q.as<int>() + q0, P.filt.queries_from(q0), s));
     KNN_CHECK(launch_export_lower(ix->ws2.thr.as<float>() + q0, ix->ws2.eps.as<float>() + q0, nb, lower_b, s));
     if (lower_j_b) {
         KNN_CHECK(launch_kth_lower(filter_state(ix->ws2, q0, P.cap), ix->ws2.eps.as<float>() + q0, nb, int(j), negate_j, lower_j_b, s));
@@ -1313,7 +1432,7 @@ static int two_phase_finish_batch(knn_index* ix, int64_t b, const float* lower_b
         // an exact shard must be finished on the same stream.
         const long long l0 = P.launches0;
         KNN_CHECK(search_dev_impl(ix, nb, row_at(P.xq, q0, ix->d, P.dtype), P.dtype, P.k, D_dev + q0 * P.k, I_dev + q0 * P.k,
-                                  id_base, s));
+                                  id_base, s, nullptr, P.filt.queries_from(q0)));
         P.launches0 = l0;
         return KNN_OK;
     }
@@ -1323,7 +1442,7 @@ static int two_phase_finish_batch(knn_index* ix, int64_t b, const float* lower_b
 static int two_phase_end(knn_index* ix, float* D_dev, int64_t* I_dev, int64_t id_base, cudaStream_t s) {
     auto& P = ix->pend;
     P.active = false;
-    if (P.tensor) KNN_CHECK(redo_overflowed(ix, P.nq, P.qb, P.nbatches, P.xq, P.dtype, P.k, D_dev, I_dev, id_base, s));
+    if (P.tensor) KNN_CHECK(redo_overflowed(ix, P.nq, P.qb, P.nbatches, P.xq, P.dtype, P.k, D_dev, I_dev, id_base, P.filt, s));
     KNN_CHECK_CUDA(cudaEventRecord(ix->search_event, s));
     if (ix->profile && ix->ev_used) {
         KNN_CHECK_CUDA(cudaStreamSynchronize(s));
@@ -1343,6 +1462,29 @@ int knn_index_search_begin_typed_dev(knn_index* ix, int64_t nq, const void* xq_d
     KNN_CHECK(two_phase_begin(ix, nq, xq_dev, dtype, k, static_cast<cudaStream_t>(stream), "search_begin"));
     *nbatches_out = ix->pend.nbatches;
     *batch_rows_out = ix->pend.qb;
+    return KNN_OK;
+}
+
+int knn_index_search_begin_params_dev(knn_index* ix, int64_t nq, const void* xq_dev, int dtype, int64_t k, int64_t id_base,
+                                      const knn_search_params* p, int64_t* nbatches_out, int64_t* batch_rows_out, void* stream) {
+    if (!ix || !nbatches_out || !batch_rows_out) {
+        set_error("search_begin: invalid arguments");
+        return KNN_ERR_INVALID;
+    }
+    DeviceGuard g(ix->device);
+    KNN_CHECK(two_phase_begin(ix, nq, xq_dev, dtype, k, static_cast<cudaStream_t>(stream), "search_begin", p, id_base));
+    *nbatches_out = ix->pend.nbatches;
+    *batch_rows_out = ix->pend.qb;
+    return KNN_OK;
+}
+
+// A filtered search's exclusion ids were read against the id base begin_params was given: the later calls repeat it.
+static int check_id_base(const knn_index* ix, int64_t id_base, const char* who) {
+    if (ix->pend.filtered && id_base != ix->pend.id_base) {
+        set_error("%s: id_base %lld differs from the %lld given to search_begin_params", who, (long long)id_base,
+                  (long long)ix->pend.id_base);
+        return KNN_ERR_INVALID;
+    }
     return KNN_OK;
 }
 
@@ -1367,6 +1509,7 @@ int knn_index_search_finish_batch_dev(knn_index* ix, int64_t b, const float* bou
         set_error("search_finish_batch: no search_begin pending, batch out of range or null output");
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_id_base(ix, id_base, "search_finish_batch"));
     DeviceGuard g(ix->device);
     const float* base = bounds_dev ? bounds_dev + b * 2 * ix->pend.qb : nullptr;
     return two_phase_finish_batch(ix, b, base, base ? base + ix->pend.qb : nullptr, D_dev, I_dev, id_base, static_cast<cudaStream_t>(stream));
@@ -1377,6 +1520,7 @@ int knn_index_search_end_dev(knn_index* ix, float* D_dev, int64_t* I_dev, int64_
         set_error("search_end: no search_begin pending");
         return KNN_ERR_INVALID;
     }
+    KNN_CHECK(check_id_base(ix, id_base, "search_end"));
     DeviceGuard g(ix->device);
     return two_phase_end(ix, D_dev, I_dev, id_base, static_cast<cudaStream_t>(stream));
 }

@@ -189,10 +189,13 @@ __device__ int block_select_sorted(const Gen& gen, int L, int k, SelectSmem& sm)
 }
 
 // ---------------------------------------------------------------------------------------
+// FILT: an ineligible row becomes the padding key 0 by its id (any score, -FLT_MAX and +FLT_MAX included, is one a row
+// can really have), so it never enters a segment list.
+template <bool FILT>
 __global__ void __launch_bounds__(kSelectThreads)
 select_dense_kernel(const float* __restrict__ scores, int64_t ld, int64_t ncols, int seg_len, uint32_t id_base, int k,
                     int largest, float* __restrict__ list_scores, uint32_t* __restrict__ list_ids, int64_t list_ld,
-                    int64_t list_off) {
+                    int64_t list_off, const RowFilter filt) {
     __shared__ SelectSmem sm;
     const int64_t q = blockIdx.y;
     const int64_t seg = blockIdx.x;
@@ -200,8 +203,19 @@ select_dense_kernel(const float* __restrict__ scores, int64_t ld, int64_t ncols,
     const int L = int((ncols - c0) < seg_len ? (ncols - c0) : seg_len);
     const float* row = scores + q * ld + c0;
     const uint32_t base = id_base + uint32_t(c0);
-    auto gen = [=] __device__(int i) { return make_key(row[i], base + uint32_t(i), largest); };
-    const int n = block_select_sorted(gen, L, k, sm);
+    int n;
+    if constexpr (FILT) {
+        const int64_t ex_row = excluded_row(filt, q);
+        auto gen = [=] __device__(int i) {
+            const uint32_t r = base + uint32_t(i);
+            if (int64_t(r) == ex_row || !row_allowed(filt, r)) return uint64_t(0);
+            return make_key(row[i], r, largest);
+        };
+        n = block_select_sorted(gen, L, k, sm);
+    } else {
+        auto gen = [=] __device__(int i) { return make_key(row[i], base + uint32_t(i), largest); };
+        n = block_select_sorted(gen, L, k, sm);
+    }
     float* os = list_scores + q * list_ld + list_off + seg * k;
     uint32_t* oi = list_ids + q * list_ld + list_off + seg * k;
     for (int r = threadIdx.x; r < k; r += blockDim.x) {
@@ -634,6 +648,11 @@ __global__ void gather_rows_kernel(const SRC* __restrict__ xq, int d, const int*
     for (int i = threadIdx.x; i < d; i += blockDim.x) dst[i] = elem_f32(src[i]);
 }
 
+__global__ void gather_ids_kernel(const int64_t* __restrict__ ids, const int* __restrict__ idx, int64_t n, int64_t* __restrict__ out) {
+    const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = ids[idx[i]];
+}
+
 __global__ void scatter_results_kernel(const float* __restrict__ Dt, const int64_t* __restrict__ It, const int* __restrict__ idx,
                                        int k, float* __restrict__ D, int64_t* __restrict__ I) {
     const int64_t q = idx[blockIdx.x];
@@ -648,15 +667,20 @@ __global__ void scatter_results_kernel(const float* __restrict__ Dt, const int64
 // ---------------------------------------------------------------------------------------
 int launch_select_dense(const float* scores, int64_t ld, int64_t ncols, int64_t nq, int seg_len, uint32_t id_base,
                         int k, int largest, float* list_scores, uint32_t* list_ids, int64_t list_ld,
-                        int64_t list_off, cudaStream_t s) {
+                        int64_t list_off, const RowFilter& filt, cudaStream_t s) {
     if (nq <= 0 || ncols <= 0) return KNN_OK;
     const int64_t nseg = (ncols + seg_len - 1) / seg_len;
     for (int64_t q0 = 0; q0 < nq; q0 += 65535) {
         const int64_t qn = nq - q0 < 65535 ? nq - q0 : 65535;
         dim3 grid((unsigned)nseg, (unsigned)qn, 1u);
-        select_dense_kernel<<<grid, kSelectThreads, 0, s>>>(scores + q0 * ld, ld, ncols, seg_len, id_base, k, largest,
-                                                            list_scores + q0 * list_ld, list_ids + q0 * list_ld,
-                                                            list_ld, list_off);
+        if (filt.active())
+            select_dense_kernel<true><<<grid, kSelectThreads, 0, s>>>(scores + q0 * ld, ld, ncols, seg_len, id_base, k, largest,
+                                                                      list_scores + q0 * list_ld, list_ids + q0 * list_ld,
+                                                                      list_ld, list_off, filt.queries_from(q0));
+        else
+            select_dense_kernel<false><<<grid, kSelectThreads, 0, s>>>(scores + q0 * ld, ld, ncols, seg_len, id_base, k, largest,
+                                                                       list_scores + q0 * list_ld, list_ids + q0 * list_ld,
+                                                                       list_ld, list_off, filt);
         KNN_CHECK_LAUNCH();
     }
     return KNN_OK;
@@ -744,6 +768,13 @@ int launch_gather_rows(const void* xq, int xq_dtype, int d, const int* idx, int6
             set_error("unknown query dtype %d", xq_dtype);
             return KNN_ERR_INVALID;
     }
+    KNN_CHECK_LAUNCH();
+    return KNN_OK;
+}
+
+int launch_gather_ids(const int64_t* ids, const int* idx, int64_t n, int64_t* out, cudaStream_t s) {
+    if (n <= 0) return KNN_OK;
+    gather_ids_kernel<<<unsigned((n + 255) / 256), 256, 0, s>>>(ids, idx, n, out);
     KNN_CHECK_LAUNCH();
     return KNN_OK;
 }

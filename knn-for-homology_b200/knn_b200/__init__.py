@@ -8,10 +8,12 @@ the reference's drivers run unchanged.
 from .index import (METRIC_INNER_PRODUCT, METRIC_L2, MAX_K, IndexFlat, IndexFlatIP, IndexFlatL2, IndexHNSWFlat,
                     IndexLSH, merge_topk, normalize_L2)
 from .io import read_index, write_index
+from .selectors import IDSelector, IDSelectorBatch, IDSelectorBitmap, IDSelectorNot, IDSelectorRange, SearchParameters
 from .postproc import (compute_auc1, compute_correctness_array, compute_is_correct, evaluate_faiss, evaluate_ids,
                        format_prefilter_db, remove_self_hit, write_prefilter_db)
 
 __all__ = ["METRIC_INNER_PRODUCT", "METRIC_L2", "MAX_K", "IndexFlat", "IndexFlatIP", "IndexFlatL2", "IndexLSH",
            "IndexHNSWFlat", "normalize_L2", "write_index", "read_index", "merge_topk", "evaluate_faiss", "evaluate_ids",
            "compute_is_correct", "compute_correctness_array", "compute_auc1", "remove_self_hit", "write_prefilter_db",
-           "format_prefilter_db"]
+           "format_prefilter_db", "SearchParameters", "IDSelector", "IDSelectorRange", "IDSelectorBatch",
+           "IDSelectorBitmap", "IDSelectorNot"]

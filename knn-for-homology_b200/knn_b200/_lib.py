@@ -21,6 +21,15 @@ DTYPE_F32 = 0
 DTYPE_F16 = 1
 DTYPE_BF16 = 2
 
+
+
+class SearchParamsC(ctypes.Structure):
+    """struct knn_search_params (filtered search)."""
+    _fields_ = [("allow_bits", c_vp), ("allow_bit0", c_i64), ("allow_nbits", c_i64), ("exclude_ids", c_vp)]
+
+
+c_params_p = ctypes.POINTER(SearchParamsC)
+
 # name -> (restype, argtypes); mirrors include/knn_b200.h one to one
 SIGNATURES = {
     "knn_last_error": (ctypes.c_char_p, []),
@@ -54,6 +63,10 @@ SIGNATURES = {
     "knn_index_search_filter_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_i64, c_vp, c_vp]),
     "knn_index_search_finish_typed_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp, c_vp, c_i64,
                                                          c_vp]),
+    "knn_index_search_params": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp, c_params_p]),
+    "knn_index_search_params_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_vp, c_vp, c_i64, c_params_p, c_vp]),
+    "knn_index_search_begin_params_dev": (ctypes.c_int, [c_vp, c_i64, c_vp, ctypes.c_int, c_i64, c_i64, c_params_p,
+                                                         ctypes.POINTER(c_i64), ctypes.POINTER(c_i64), c_vp]),
     "knn_index_reconstruct": (ctypes.c_int, [c_vp, c_i64, c_i64, c_vp]),
     "knn_merge_topk_dev": (ctypes.c_int, [ctypes.c_int, c_i64, c_i64, ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "knn_peer_buffer_alloc": (ctypes.c_int, [ctypes.POINTER(c_vp), c_i64, ctypes.c_int]),

@@ -431,11 +431,17 @@ class ShardedIndexFlat:
         self._dist.all_gather_into_tensor(buf, mine, group=self.group)
         return buf[:n]
 
-    def search(self, x, k: int):
+    def search(self, x, k: int, *, params=None, exclude=None):
         """Returns the merged (D, I) on every rank (torch tensors on the local index's device, or
         numpy arrays when x is numpy).  Calls with more queries than the two-phase search keeps resident
-        (TWO_PHASE_MAX_QUERIES) are processed in chunks of that size (config C5: 1M queries)."""
+        (TWO_PHASE_MAX_QUERIES) are processed in chunks of that size (config C5: 1M queries).
+
+        params (faiss.SearchParameters(sel=...)) selects global rows and exclude (an (nq,) array of global ids, -1:
+        none) removes one row per query; a filtered search always runs the pipelined two-phase search, every shard
+        reading the one global bitmap from its first global row on."""
         n = x.shape[0]
+        if (getattr(params, "sel", None) is not None or exclude is not None) and n > 0:
+            return self._search_filtered(x, k, params, exclude)
         if n == 0:  # nothing to search (every rank of the group sees the same empty call: no collective is entered)
             if isinstance(x, np.ndarray):
                 return np.empty((0, k), np.float32), np.empty((0, k), np.int64)
@@ -530,7 +536,40 @@ class ShardedIndexFlat:
             return _to_numpy(D), _to_numpy(I)
         return D, I
 
-    def _two_phase_pipelined(self, xd, k: int, mark):
+    def _search_filtered(self, x, k: int, params, exclude):
+        import torch
+
+        if len(self._segments) > 1:
+            raise NotImplementedError("a filtered search of a ShardedIndexFlat needs its rows from a single add()")
+        as_numpy = isinstance(x, np.ndarray)
+        dev = torch.device("cuda", self.local.device) if torch.cuda.is_available() else torch.device("cpu")
+        on_cuda = self._dist.is_initialized() and self._dist.get_backend(self.group) == "nccl"
+        xd = self.upload_queries(x) if on_cuda and (as_numpy or not x.is_cuda) else torch.as_tensor(x).to(dev)
+        g0 = self._segments[0][0] if self._segments else 0
+        if exclude is not None:
+            exclude = torch.as_tensor(exclude, dtype=torch.int64).to(dev)
+        flt = {"params": params, "exclude": exclude, "id_base": g0, "allow_bit0": g0, "allow_nbits": self._ntotal}
+        parts = []
+        for i in range(0, xd.shape[0], self.TWO_PHASE_MAX_QUERIES):
+            sl = slice(i, i + self.TWO_PHASE_MAX_QUERIES)
+            chunk = dict(flt, exclude=exclude[sl] if exclude is not None else None)
+            D, I = self._two_phase_pipelined(xd[sl], k, lambda *a: None, chunk)
+            if self.world > 1 and self.peer_merge and D.is_cuda and self.world <= 16 and (self.world + 1) * k * 8 <= 200 * 1024:
+                D, I = self._merge_over_peer_memory(D, I)
+            elif self.world > 1:
+                nq, kk = D.shape
+                Dg = torch.empty((self.world * nq, kk), dtype=D.dtype, device=D.device)
+                Ig = torch.empty((self.world * nq, kk), dtype=I.dtype, device=I.device)
+                self._dist.all_gather_into_tensor(Dg, D.contiguous(), group=self.group)
+                self._dist.all_gather_into_tensor(Ig, I.contiguous(), group=self.group)
+                D, I = self._merge(Dg.view(self.world, nq, kk), Ig.view(self.world, nq, kk), self.metric_type)
+            parts.append((D, I))
+        D, I = (torch.cat([p[0] for p in parts]), torch.cat([p[1] for p in parts])) if len(parts) > 1 else parts[0]
+        if as_numpy:
+            return _to_numpy(D), _to_numpy(I)
+        return D, I
+
+    def _two_phase_pipelined(self, xd, k: int, mark, flt=None):
         """The two-phase search, one query batch at a time over two streams.  Main stream: tensor-core filter of
         batch 0, 1, 2 ...  Side stream, per batch as soon as its filter is done: ONE all-reduce(MAX) of the batch's two
         bounds (a few hundred KB over NVLink), then the finish phase (exact rescoring of what can still be in the
@@ -551,12 +590,14 @@ class ShardedIndexFlat:
         nq = xd.shape[0]
         main.wait_stream(caller)
         with torch.cuda.stream(main):
-            nbatches, rows = self.local.search_begin(xd, k)
+            nbatches, rows = self.local.search_begin(xd, k, **flt) if flt else self.local.search_begin(xd, k)
             bx = self._bounds_exchange(nbatches, rows) if self.peer_bounds else None
             bounds = torch.zeros((nbatches, 2, rows), dtype=torch.float32, device=dev)
             D = torch.empty((nq, k), dtype=torch.float32, device=dev)
             I = torch.empty((nq, k), dtype=torch.int64, device=dev)
             id_base = self._segments[0][0] if len(self._segments) == 1 else 0
+            if flt:
+                id_base = flt["id_base"]
             j = -(-k // self.world)
             side.wait_stream(main)  # bounds / D / I exist before the side stream touches them
             for b in range(nbatches):
@@ -726,9 +767,12 @@ class GridIndexFlat:
         b = self.query_bounds(n)
         return b[self.g], b[self.g + 1]
 
-    def search(self, x, k: int):
+    def search(self, x, k: int, *, params=None, exclude=None):
         """Every rank passes ALL queries and gets the full (D, I); its group searches rows [lo, hi) of them."""
         import torch
+
+        if getattr(params, "sel", None) is not None or exclude is not None:
+            raise NotImplementedError("GridIndexFlat has no filtered search; use ShardedIndexFlat (row shards only)")
 
         as_numpy = isinstance(x, np.ndarray)
         n = x.shape[0]

@@ -199,8 +199,57 @@ class IndexFlat:
     def reset(self) -> None:
         _lib.check(self._lib.knn_index_reset(self._h))
 
-    def search(self, x, k: int, id_base: int = 0):
-        """(D, I) of the k best rows per query, best first (cath/search.py:24)."""
+    def _search_params(self, params, exclude, nq: int, id_base: int, on_device: bool, allow_bit0: int = 0,
+                       allow_nbits: int | None = None):
+        """(knn_search_params or None, the arrays it points to).  params.sel becomes one packed bitmap (built on the
+        device for a device search, on the host for a host search; allow_nbits defaults to ntotal); exclude, an (nq,)
+        array of ids in the space the call returns (-1: none), is passed as int64 - for a host search with the id base
+        taken off, because the host call returns row numbers and the id base is added afterwards."""
+        sel = getattr(params, "sel", None) if params is not None else None
+        if sel is None and exclude is None:
+            return None, ()
+        if allow_nbits is None:
+            allow_nbits = self.ntotal
+        c = _lib.SearchParamsC(None, int(allow_bit0), int(allow_nbits), None)
+        keep = []
+        if on_device:
+            import torch
+
+            dev = torch.device("cuda", self.device)
+            if sel is not None:
+                bits = sel.bitmap(int(allow_nbits), device=dev)
+                keep.append(bits)
+                c.allow_bits = bits.data_ptr()
+            if exclude is not None:
+                ex = torch.as_tensor(exclude, dtype=torch.int64).to(dev).contiguous().view(-1)
+                if ex.shape[0] != nq:
+                    raise ValueError("exclude must hold one id per query (%d), got %d" % (nq, ex.shape[0]))
+                keep.append(ex)
+                c.exclude_ids = ex.data_ptr()
+        else:
+            if sel is not None:
+                bits = np.ascontiguousarray(sel.bitmap(int(allow_nbits)))
+                keep.append(bits)
+                c.allow_bits = bits.ctypes.data
+            if exclude is not None:
+                ex = exclude.detach().cpu().numpy() if _is_torch(exclude) else exclude
+                ex = np.ascontiguousarray(np.asarray(ex, dtype=np.int64).reshape(-1))
+                if ex.shape[0] != nq:
+                    raise ValueError("exclude must hold one id per query (%d), got %d" % (nq, ex.shape[0]))
+                if id_base:
+                    ex = np.ascontiguousarray(np.where(ex >= int(id_base), ex - int(id_base), -1))
+                keep.append(ex)
+                c.exclude_ids = ex.ctypes.data
+        keep.append(c)
+        return c, keep
+
+    def search(self, x, k: int, id_base: int = 0, *, params=None, exclude=None):
+        """(D, I) of the k best rows per query, best first (cath/search.py:24).
+
+        params: faiss.SearchParameters(sel=IDSelector...) restricts the search to the selected rows.  exclude (an
+        extension): an (nq,) array or tensor of ids, -1 for none; id exclude[q] is never returned for query q (ids
+        include id_base).  A filtered search returns exactly what an unfiltered one returns on an index of the
+        eligible rows alone, ids mapped back; queries with fewer than k eligible rows get id -1 padding."""
         k = int(k)
         if k <= 0:
             raise ValueError("k must be positive")
@@ -210,12 +259,23 @@ class IndexFlat:
             x, code = self._dev_matrix(x)
             D = torch.empty((x.shape[0], k), dtype=torch.float32, device=x.device)
             I = torch.empty((x.shape[0], k), dtype=torch.int64, device=x.device)
-            _lib.check(self._lib.knn_index_search_typed_dev(self._h, x.shape[0], x.data_ptr(), code, k, D.data_ptr(),
-                                                            I.data_ptr(), int(id_base), _torch_stream(self.device)))
+            p, keep = self._search_params(params, exclude, x.shape[0], id_base, on_device=True)
+            if p is None:
+                _lib.check(self._lib.knn_index_search_typed_dev(self._h, x.shape[0], x.data_ptr(), code, k, D.data_ptr(),
+                                                                I.data_ptr(), int(id_base), _torch_stream(self.device)))
+            else:  # the filter arrays are read on the current stream, which later frees of them are ordered behind
+                _lib.check(self._lib.knn_index_search_params_dev(self._h, x.shape[0], x.data_ptr(), code, k, D.data_ptr(),
+                                                                 I.data_ptr(), int(id_base), ctypes.byref(p),
+                                                                 _torch_stream(self.device)))
             return D, I
         x, code, ptr = self._host_rows(x)
         D, I = _result_arrays(x.shape[0], k)
-        _lib.check(self._lib.knn_index_search_typed(self._h, x.shape[0], ptr, code, k, D.ctypes.data, I.ctypes.data))
+        p, keep = self._search_params(params, exclude, x.shape[0], id_base, on_device=False)
+        if p is None:
+            _lib.check(self._lib.knn_index_search_typed(self._h, x.shape[0], ptr, code, k, D.ctypes.data, I.ctypes.data))
+        else:
+            _lib.check(self._lib.knn_index_search_params(self._h, x.shape[0], ptr, code, k, D.ctypes.data, I.ctypes.data,
+                                                         ctypes.byref(p)))
         if id_base:
             I[I >= 0] += int(id_base)
         return D, I
@@ -253,13 +313,25 @@ class IndexFlat:
         return D, I
 
     # -- the same, batch by batch (the caller overlaps exchange + finish of batch b with the filter of batch b + 1) --
-    def search_begin(self, x, k: int):
-        """Returns (nbatches, batch_rows); x is kept alive until search_end."""
+    def search_begin(self, x, k: int, params=None, exclude=None, id_base: int = 0, allow_bit0: int = 0,
+                     allow_nbits: int | None = None):
+        """Returns (nbatches, batch_rows); x (and the filter) are kept alive until search_end.  With params / exclude
+        the batches are filtered (see search); finish_batch and end must then be given the same id_base.  A shard of a
+        row-sharded database passes the global selector with allow_bit0 = its first global row and allow_nbits = the
+        global row count."""
         x, code = self._dev_matrix(x)
         nb, rows = ctypes.c_int64(), ctypes.c_int64()
-        _lib.check(self._lib.knn_index_search_begin_typed_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
-                                                              ctypes.byref(nb), ctypes.byref(rows), _torch_stream(self.device)))
+        p, keep = self._search_params(params, exclude, x.shape[0], id_base, on_device=True, allow_bit0=allow_bit0,
+                                      allow_nbits=allow_nbits)
+        if p is None:
+            _lib.check(self._lib.knn_index_search_begin_typed_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
+                                                                  ctypes.byref(nb), ctypes.byref(rows), _torch_stream(self.device)))
+        else:
+            _lib.check(self._lib.knn_index_search_begin_params_dev(self._h, x.shape[0], x.data_ptr(), code, int(k),
+                                                                   int(id_base), ctypes.byref(p), ctypes.byref(nb),
+                                                                   ctypes.byref(rows), _torch_stream(self.device)))
         self._pending_x = x
+        self._pending_filter = keep
         return nb.value, rows.value
 
     def search_filter_batch(self, b: int, j: int, bounds) -> None:
@@ -273,6 +345,7 @@ class IndexFlat:
     def search_end(self, D, I, id_base: int = 0) -> None:
         _lib.check(self._lib.knn_index_search_end_dev(self._h, D.data_ptr(), I.data_ptr(), int(id_base), _torch_stream(self.device)))
         self._pending_x = None
+        self._pending_filter = ()
 
     def search_into(self, xq_ptr: int, nq: int, k: int, D_ptr: int, I_ptr: int, dtype: int = _lib.DTYPE_F32) -> None:
         """Host-pointer search into caller-owned (e.g. pinned) buffers: the raw C-ABI call (dtype: a KNN_DTYPE code)."""
